@@ -14,6 +14,11 @@ render  : secondary number — rendered rays/s of BASELINE.json cfg 3 (1008x756 
           rays sharded over the GPUs with one final gather.
 roofline: the kernel with the largest share of the step, timed with CUDA events inside the timed region.
 One JSON line on stdout (rank 0).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed training step left its caller, as float32
+DIR/<name>.npy: `loss` (the value the step returns), and for both networks `param.<net>.<tensor>` (the weights after that step's Adam update) and
+`grad.<net>.<tensor>` (the gradients it applied), about 10 MB in all.  Rays, targets, initial weights and random draws are
+seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -297,6 +302,19 @@ def kernel_table():
             "head_grads_kernel": (0, HBM_HEADS, "read")}
 
 
+def dump_outputs(out_dir, loss, nets):
+    """--dump-outputs: the loss of the last step and, per network, its updated parameters and the gradients it applied."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    for net_name, net in nets.items():
+        for name, p in net.named_parameters():
+            name = net_name + "." + name.replace("module.", "")
+            arrays["param." + name] = p
+            arrays["grad." + name] = p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(a):
     global N_RAND
     N_RAND = int(a.rays_per_gpu)
@@ -392,8 +410,14 @@ def run_ours(a):
         resident_step()                        # (all ranks: the step contains a collective)
     torch.cuda.synchronize()
     clocks.mark()
-    ms_total = timed(resident_step, a.steps)
+    last = {}
+
+    def timed_step():
+        last["loss"] = resident_step()
+    ms_total = timed(timed_step, a.steps)
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:       # before the sections below train the networks further
+        dump_outputs(a.dump_outputs, last["loss"], {"coarse": coarse, "fine": fine})
     ms_step = ms_total / a.steps
     value = world * N_RAND / (ms_step * 1e-3)
 
@@ -608,8 +632,14 @@ def main():
     ap.add_argument("--overlap-allreduce", action="store_true",
                     help="start each network's gradient allreduce from autograd hooks while the backward still runs (default: after it)")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, parameters and gradients of the last timed step to DIR/<name>.npy (product arm)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
+        if a.dump_outputs:
+            ap.error("--dump-outputs writes what the product arm computed; the reference arm has none")
         os.environ["CUDA_VISIBLE_DEVICES"] = ""      # the reference picks `cuda` when it sees one (run.py:46): this arm is its CPU path
         run_reference(a)
     else:

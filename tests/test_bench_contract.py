@@ -1,10 +1,13 @@
 """CPU suite: the reference arm of bench.py (the unmodified reference staged under oracle/_ref — or /root/reference — on the
 host cores; the CPU port only where neither exists) runs here and prints ONE JSON line with the contract's keys; the product
-arm refuses to run without a CUDA device (no CPU fallback)."""
+arm refuses to run without a CUDA device (no CPU fallback).  On a GPU, the product arm's --dump-outputs is checked."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -55,3 +58,22 @@ def test_product_arm_has_no_cpu_fallback():
         return
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1"], capture_output=True, text=True, timeout=300)
     assert p.returncode != 0 and "no CPU fallback" in (p.stderr + p.stdout)
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_the_last_timed_step(tmp_path):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert p.returncode == 0, p.stderr[-2000:]
+    d = json.loads([ln for ln in p.stdout.splitlines() if ln.startswith("{")][-1])
+    assert d["steps"] == 2
+    files = sorted(tmp_path.glob("*.npy"))
+    assert sum(f.stat().st_size for f in files) <= 64 << 20
+    out = {f.stem: np.load(f) for f in files}
+    assert all(v.dtype in (np.float32, np.float64) and np.isfinite(v).all() for v in out.values())
+    assert float(out["loss"]) > 0
+    params = [k[len("param."):] for k in out if k.startswith("param.")]
+    assert len(params) == 48 and sorted(params) == sorted(k[len("grad."):] for k in out if k.startswith("grad."))
+    assert len(out) == 1 + 2 * len(params)
+    for k in params:
+        assert out["param." + k].shape == out["grad." + k].shape and np.abs(out["grad." + k]).max() > 0, k
