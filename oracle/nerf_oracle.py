@@ -514,16 +514,18 @@ def bf16_round(x):
     return a.astype(np.uint32).view(np.float32).reshape(np.shape(x)).astype(np.float64)
 
 
-def nerf_forward_backward_bf16sim(p, pts, viewdirs, d_out=None, multires=10, multires_views=4):
+def nerf_forward_backward_bf16sim(p, pts, viewdirs, d_out=None, multires=10, multires_views=4, keep=False):
     """Forward (and, with d_out, backward) of the NeRF MLP with every tensor-core operand rounded to
     bf16 exactly where the kernels round: MMA weights, PE inputs, each layer's activation, each dZ.
-    The alpha / rgb heads run on fp32 activations with fp32 weights, as in mlp_forward.cu."""
+    The alpha / rgb heads run on fp32 activations with fp32 weights, as in mlp_forward.cu.
+    keep=True appends a dict of the intermediates: pe, vpe, ins / pre / h (input, pre-activation and bf16 output of each
+    pts_linears layer), feat, pre_v, hidden (bf16), and with d_out d_hidden_pre, d_feat and dz (dZ of each pts_linears layer)."""
     W = {k: (bf16_round(v) if (k.endswith("weight") and not k.startswith(("alpha", "rgb"))) else v.astype(np.float64))
          for k, v in p.items()}
     pe = bf16_round(embed(pts, multires))
     vpe = bf16_round(embed(viewdirs, multires_views))
     h = pe
-    ins, pre = [], []
+    ins, pre, outs = [], [], []
     h8_f = None
     for i in range(8):
         ins.append(h)
@@ -531,6 +533,7 @@ def nerf_forward_backward_bf16sim(p, pts, viewdirs, d_out=None, multires=10, mul
         pre.append(z)
         hf = np.maximum(z, 0)
         h = bf16_round(hf)
+        outs.append(h)
         if i == 7:
             h8_f = hf
         if i == 4:
@@ -543,8 +546,9 @@ def nerf_forward_backward_bf16sim(p, pts, viewdirs, d_out=None, multires=10, mul
     hv_f = np.maximum(pre_v, 0)
     rgb = hv_f @ W["rgb_linear.weight"].T + W["rgb_linear.bias"]
     out = np.concatenate([rgb, alpha], -1)
+    saved = dict(pe=pe, vpe=vpe, ins=ins, pre=pre, h=outs, feat=feat, pre_v=pre_v, hidden=bf16_round(hv_f))
     if d_out is None:
-        return out
+        return (out, saved) if keep else out
     g = {}
     d_out = np.asarray(d_out, dtype=np.float64)
     d_rgb, d_alpha = d_out[:, :3], d_out[:, 3:4]
@@ -560,13 +564,17 @@ def nerf_forward_backward_bf16sim(p, pts, viewdirs, d_out=None, multires=10, mul
     g["feature_linear.weight"] = d_feat.T @ h8
     g["feature_linear.bias"] = d_feat.sum(0)
     d_h = d_feat @ W["feature_linear.weight"] + d_alpha @ W["alpha_linear.weight"]
+    dz = [None] * 8
     for i in reversed(range(8)):
         if i == 4:
             d_h = d_h[:, 63:]
-        d_pre = bf16_round(d_h * (pre[i] > 0))
+        d_pre = dz[i] = bf16_round(d_h * (pre[i] > 0))
         g["pts_linears.%d.weight" % i] = d_pre.T @ ins[i]
         g["pts_linears.%d.bias" % i] = d_pre.sum(0)
         d_h = d_pre @ W["pts_linears.%d.weight" % i]
+    if keep:
+        saved.update(d_hidden_pre=d_pre_v, d_feat=d_feat, dz=dz)
+        return out, g, saved
     return out, g
 
 

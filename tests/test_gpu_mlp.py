@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 import torch
 
+import mlp_ref64 as ref
 from oracle import nerf_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -116,76 +117,10 @@ GRAD_TF_RTOL = 5e-3
 GRAD_REF_COS = 0.99
 GRAD_REF_RTOL = 0.25
 
-_IMG_IDX = None
-
-
-def _img_index():
-    """byte offset -> (row, col) gather index of a 128x64 bf16 chunk image (128-byte swizzle)."""
-    global _IMG_IDX
-    if _IMG_IDX is None:
-        r = np.arange(128)[:, None]
-        k = np.arange(64)[None, :]
-        off = (r >> 3) * 1024 + (r & 7) * 128 + ((((k >> 3) ^ (r & 7))) << 4) + (k & 7) * 2
-        _IMG_IDX = (off // 2).astype(np.int64)
-    return _IMG_IDX
-
-
-def decode_stash(stash, P):
-    """-> dict of float64 arrays [P, feat] and bool masks, from the forward stash bytes."""
-    buf = stash.cpu().numpy()
-    tile_bytes = 40 * 16384 + 9 * 128 * 32
-    T = (P + 127) // 128
-    idx = _img_index()
-    out = {k: [] for k in ("pe", "h", "feat", "vpe", "hidden", "mask")}
-    for t in range(T):
-        tb = buf[t * tile_bytes:(t + 1) * tile_bytes]
-        imgs = tb[:40 * 16384].view(np.uint16).reshape(40, 8192)
-        dec = (imgs[:, idx].astype(np.uint32) << 16).view(np.float32).astype(np.float64)     # [40,128,64]
-        out["pe"].append(dec[0])
-        out["h"].append(np.stack([np.concatenate(list(dec[1 + 4 * l:5 + 4 * l]), -1) for l in range(8)], 0))
-        out["feat"].append(np.concatenate(list(dec[33:37]), -1))
-        out["vpe"].append(dec[37])
-        out["hidden"].append(np.concatenate(list(dec[38:40]), -1))
-        # [layer][column half ch][row][N-half h][2 words] -> [layer][row][word 2 (2 h + ch) + i]   (mlp_common.cuh)
-        m = tb[40 * 16384:].view(np.uint32).reshape(9, 2, 128, 2, 2).transpose(0, 2, 3, 1, 4).reshape(9, 128, 8)
-        j = np.arange(32)
-        bitpos = (16 * (j & 1) + 8 * (j >> 4) + ((j & 15) >> 1)).astype(np.uint32)     # mask_bit_of_column (mlp_common.cuh)
-        bits = ((m[..., None] >> bitpos) & 1).astype(bool).reshape(9, 128, 256)
-        out["mask"].append(bits)
-    res = {"pe": np.concatenate(out["pe"], 0)[:P], "feat": np.concatenate(out["feat"], 0)[:P],
-           "vpe": np.concatenate(out["vpe"], 0)[:P], "hidden": np.concatenate(out["hidden"], 0)[:P],
-           "h": np.concatenate(out["h"], 1)[:, :P], "mask": np.concatenate(out["mask"], 1)[:, :P]}
-    return res
-
-
-def teacher_forced_grads(p, st, d_out):
-    """float64 backward from the decoded stash, rounding dZ to bf16 where the dgrad chain does."""
-    bf = orc.bf16_round
-    W = {k: bf(v) if k.endswith("weight") else v.astype(np.float64) for k, v in p.items()}
-    d_out = np.asarray(d_out, dtype=np.float64)
-    d_rgb, d_alpha = d_out[:, :3], d_out[:, 3:4]
-    g = {}
-    g["rgb_linear.weight"] = d_rgb.T @ st["hidden"]
-    g["rgb_linear.bias"] = d_rgb.sum(0)
-    g["alpha_linear.weight"] = d_alpha.T @ st["h"][7]
-    g["alpha_linear.bias"] = d_alpha.sum(0)
-    d_pre_v = bf((d_rgb @ p["rgb_linear.weight"].astype(np.float64)) * st["mask"][8][:, :128])
-    g["views_linears.0.weight"] = d_pre_v.T @ np.concatenate([st["feat"], st["vpe"][:, :27]], -1)
-    g["views_linears.0.bias"] = d_pre_v.sum(0)
-    d_feat = bf(d_pre_v @ W["views_linears.0.weight"][:, :256])
-    g["feature_linear.weight"] = d_feat.T @ st["h"][7]
-    g["feature_linear.bias"] = d_feat.sum(0)
-    d_h = d_feat @ W["feature_linear.weight"] + d_alpha @ p["alpha_linear.weight"].astype(np.float64)
-    for i in reversed(range(8)):
-        d_pre = bf(d_h * st["mask"][i])
-        x_in = st["pe"][:, :63] if i == 0 else st["h"][i - 1]
-        if i == 5:
-            x_in = np.concatenate([st["pe"][:, :63], x_in], -1)
-        g["pts_linears.%d.weight" % i] = d_pre.T @ x_in
-        g["pts_linears.%d.bias" % i] = d_pre.sum(0)
-        Wi = W["pts_linears.%d.weight" % i]
-        d_h = d_pre @ (Wi[:, 63:] if i == 5 else Wi)
-    return g
+def teacher_forced_grads(p, stash, P, d_out):
+    """float64 backward from the decoded stash, rounding dZ to bf16 where the dgrad chain does (mlp_ref64)"""
+    g = ref.teacher_forced_grads(p, stash, P, torch.as_tensor(np.asarray(d_out, dtype=np.float32)))
+    return {n: v.cpu().numpy() for n, v in g.items()}
 
 
 def _check_grads(ops, got, want_by_name, P, teacher_forced):
@@ -213,7 +148,7 @@ def test_mlp_backward_vs_reference_autograd(ops, golden):
     raw, stash = ops.mlp_forward(blob, pts=emb[:, 0:3], dirs=emb[:, 63:66], want_stash=True)
     grads = ops.mlp_backward(blob, cu(fx["d_out"]), stash)
     _check_grads(ops, grads, {n: fx["grad." + n] for n in ops.PARAM_ORDER}, P, teacher_forced=False)
-    _check_grads(ops, grads, teacher_forced_grads(p, decode_stash(stash, P), fx["d_out"]), P, teacher_forced=True)
+    _check_grads(ops, grads, teacher_forced_grads(p, stash, P, fx["d_out"]), P, teacher_forced=True)
     # accumulate=True adds on top
     grads2 = ops.mlp_backward(blob, cu(fx["d_out"]), stash, grads=[g.clone() for g in grads], accumulate=True)
     for a, b in zip(grads, grads2):
@@ -228,12 +163,14 @@ def test_stash_matches_bf16_model(ops):
     pts = ((rng.rand(P, 3) * 2 - 1) * 5).astype(np.float32)
     vd = rng.randn(P, 3).astype(np.float32)
     raw, stash = ops.mlp_forward(pack(ops, p), pts=cu(pts), dirs=cu(vd), want_stash=True)
-    st = decode_stash(stash, P)
+    st = ref.decode_stash(stash, P, range(ref.num_tiles(P)))
+    st = {k: [x[:P].cpu().numpy() for x in v] if isinstance(v, list) else v[:P].cpu().numpy() for k, v in st.items() if k != "finite"}
     np.testing.assert_allclose(st["pe"][:, :63], orc.bf16_round(orc.embed(pts, 10)), atol=8e-3)   # 1 bf16 ulp at |x|<=1... sin/cos
     np.testing.assert_allclose(st["vpe"][:, :27], orc.bf16_round(orc.embed(vd, 4)), atol=2e-2)
     assert np.all(st["pe"][:, 63] == 0) and np.all(st["vpe"][:, 27:] == 0)
-    assert np.array_equal(st["mask"][:8], st["h"] > 0)               # bit masks == sign of the stored activations
-    assert np.array_equal(st["mask"][8][:, :128], st["hidden"] > 0)
+    for l in range(8):
+        assert np.array_equal(st["mask"][l], st["h"][l] > 0)         # bit masks == sign of the stored activations
+    assert np.array_equal(st["mask"][8], st["hidden"] > 0)
     out_m = orc.nerf_forward_backward_bf16sim(p, pts, vd)
     assert np.abs(raw.cpu().numpy() - out_m).max() < 2e-3
 
@@ -249,7 +186,7 @@ def test_mlp_backward_ragged_sizes_vs_oracle(ops, P):
     blob = pack(ops, p)
     raw, stash = ops.mlp_forward(blob, pts=cu(pts), dirs=cu(vd), want_stash=True)
     grads = ops.mlp_backward(blob, cu(d_out), stash)
-    _check_grads(ops, grads, teacher_forced_grads(p, decode_stash(stash, P), d_out), P, teacher_forced=True)
+    _check_grads(ops, grads, teacher_forced_grads(p, stash, P, d_out), P, teacher_forced=True)
     if P >= 1000:
         x = np.concatenate([orc.embed(pts, 10), orc.embed(vd, 4)], -1)
         _, saved = orc.nerf_forward(p, x, keep=True, dtype=np.float64)
