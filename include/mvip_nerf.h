@@ -63,6 +63,21 @@ int mvip_rays_from_pose_ndc(const float* c2w, const float* c2w_static, int H, in
 int mvip_rays_pack(const float* rays_o, const float* rays_d, const float* view_d, int64_t n, float near, float far,
                    int use_viewdirs, int ndc, int H, int W, double focal, double ndc_near, float* out, void* stream);
 
+/* Backward of the two entries above (autograd of the reference's fp32 formulas, in fp32): g_out [n, 8 + 3*use_viewdirs] is the
+ * gradient of the packed batch; the near / far columns carry none.
+ *   mvip_rays_pack_backward: -> g_rays_o, g_rays_d [n,3] (overwritten); g_view_d [n,3] when view_d is given (else the view
+ *     vectors' gradient is added to g_rays_d).
+ *   mvip_rays_from_pose_backward: -> g_c2w [3,4] (overwritten); with c2w_static (then g_c2w_static is required, and only then),
+ *     g_c2w gets the view-direction part and g_c2w_static [3,4] the rays_o / rays_d part.  Bitwise reproducible: per-block partials in `workspace`
+ *     (mvip_rays_from_pose_backward_workspace_bytes()) summed in a fixed order.  Two launches. */
+int mvip_rays_pack_backward(const float* rays_o, const float* rays_d, const float* view_d, int64_t n, int use_viewdirs, int ndc,
+                            int H, int W, double focal, double ndc_near, const float* g_out, float* g_rays_o, float* g_rays_d,
+                            float* g_view_d, void* stream);
+size_t mvip_rays_from_pose_backward_workspace_bytes(void);
+int mvip_rays_from_pose_backward(const float* c2w, const float* c2w_static, int H, int W, double focal, int i0, int j0, int h,
+                                 int w, int use_viewdirs, int ndc, double ndc_near, const float* g_out, float* g_c2w,
+                                 float* g_c2w_static, void* workspace, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Stratified sampling along rays.            replaces DS_NeRF/run.py:1759-1781 (render_rays)
  *   rays    [n_rays, ray_stride] fp32: o(0:3) d(3:6) near(6) far(7) ...
@@ -135,6 +150,16 @@ int mvip_composite_backward_mse(const float* raw, const float* z_vals, const flo
                                 const float* target_rgb, const float* target_disp, const float* g_sq, const float* g_rgb,
                                 const float* g_disp, const float* g_acc, const float* g_depth, const float* g_weights,
                                 const float* g_alpha, float* d_raw, void* stream);
+
+/* mvip_composite_backward[_mse] that also differentiates the ray directions: d_rays_d [n,3] (overwritten) =
+ * d|rays_d| * rays_d / |rays_d|, d|rays_d| = sum_s dalpha_s relu(sigma_s) dist_s exp(-relu(sigma_s) dist_s |rays_d|) (last dist
+ * 1e10, as in the reference).  target_rgb / target_disp / g_sq as in mvip_composite_backward_mse, or all NULL for the plain form.
+ * d_raw is bitwise equal to that of the entry without d_rays_d. */
+int mvip_composite_backward_rays(const float* raw, const float* z_vals, const float* rays_d, int rays_d_stride,
+                                 const float* noise, int64_t n_rays, int n_samples, int white_bkgd, int detach_weights,
+                                 const float* target_rgb, const float* target_disp, const float* g_sq, const float* g_rgb,
+                                 const float* g_disp, const float* g_acc, const float* g_depth, const float* g_weights,
+                                 const float* g_alpha, float* d_raw, float* d_rays_d, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Depth -> least-squares plane normal.       replaces DS_NeRF/run.py:1909-1940
@@ -222,6 +247,13 @@ int mvip_mlp_backward(const void* packed, const float* d_raw /* [n_points,4] */,
  * kernel with its own events; phases must run in order on the same workspace. */
 int mvip_mlp_backward_phases(const void* packed, const float* d_raw, int64_t n_points, const void* stash,
                              void* workspace, float* const* grads, int accumulate, int phase_mask, void* stream);
+
+/* Gradient with respect to the MLP's inputs, from the dZ images a completed mvip_mlp_backward left in `bwd_workspace` (same
+ * stream, same packed weights, same points).  Points mode: d_points [n_points,6] = (d pts | d dirs).  Rays mode: d_points is a
+ * [n_points,6] scratch and d_rays [n_rays, ray_stride] (overwritten, every column) receives d o = sum_s d pts, d d = sum_s z_s d pts
+ * in columns 0:6 and d viewdir in viewdir_offset:+3 (fixed-order sums: bitwise reproducible).  z_vals get no gradient. */
+int mvip_mlp_input_grad(const void* packed, const mvip_points* pts, const void* bwd_workspace, float* d_points, float* d_rays,
+                        void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Self tests of the tcgen05 building blocks (descriptor / layout conventions), used by tests/.

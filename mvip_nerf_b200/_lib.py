@@ -30,6 +30,11 @@ _SIGNATURES = {
                                         c_int, c_int, c_double, c_void_p, c_void_p]),
     "mvip_rays_pack": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_float, c_float, c_int, c_int, c_int, c_int, c_double,
                                c_double, c_void_p, c_void_p]),
+    "mvip_rays_pack_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_double, c_double,
+                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mvip_rays_from_pose_backward_workspace_bytes": (c_size_t, []),
+    "mvip_rays_from_pose_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_int, c_int, c_int, c_int, c_int, c_int,
+                                             c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "mvip_sample_coarse": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "mvip_sample_pdf": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_void_p,
                                 c_void_p, c_void_p]),
@@ -46,6 +51,9 @@ _SIGNATURES = {
     "mvip_composite_backward_mse": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int, c_void_p,
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                             c_void_p]),
+    "mvip_composite_backward_rays": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int, c_void_p,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                             c_void_p, c_void_p]),
     "mvip_normal_workspace_bytes": (c_size_t, [c_int, c_int]),
     "mvip_normal_forward": (c_int, [c_void_p, c_int, c_int, c_float, c_float, c_float, c_float, c_int, c_void_p,
                                     c_void_p, c_void_p]),
@@ -67,6 +75,7 @@ _SIGNATURES = {
                                   c_void_p]),
     "mvip_mlp_backward_phases": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, POINTER(c_void_p), c_int,
                                          c_int, c_void_p]),
+    "mvip_mlp_input_grad": (c_int, [c_void_p, POINTER(MvipPoints), c_void_p, c_void_p, c_void_p, c_void_p]),
     "mvip_debug_profile": (c_int, [c_void_p]),
     "mvip_debug_trace": (c_int, [c_void_p, c_void_p]),
     "mvip_debug_wgrad_profile": (c_int, [c_void_p]),

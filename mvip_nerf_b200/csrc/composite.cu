@@ -132,13 +132,18 @@ composite_fwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
   }
 }
 
-template <int C>
+// kNorm: also d |rays_d| = sum_s dalpha_s relu(sigma_s) dist_s exp(-relu(sigma_s) dist_s |d|), chained to d rays_d [n,3] (d_dir);
+// the last dist is 1e10 as in the reference.  The sum is formed with delta_s = dist_s |d| (already in registers) and divided by
+// |d| once: d rays_d = (sum_s dalpha_s relu(sigma_s) delta_s e_s) d / |d|^2 (0 when |d| = 0).  relu(sigma) multiplies rather
+// than selects, so a NaN dalpha (a ray whose every sigma <= 0: disp = 1/max(1e-10, 0/0)) gives NaN, as the reference's autograd
+// does through dists.  d_raw does not depend on the flag.
+template <int C, bool kNorm>
 __global__ void __launch_bounds__(kWarps * 32)
 composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z, const float* __restrict__ rays_d,
                      int d_stride, const float* __restrict__ noise, int64_t n_rays, int S, int white, int detach_w,
                      const float* __restrict__ g_rgb, const float* __restrict__ g_disp, const float* __restrict__ g_acc,
                      const float* __restrict__ g_depth, const float* __restrict__ g_weights,
-                     const float* __restrict__ g_alpha, float4* __restrict__ d_raw) {
+                     const float* __restrict__ g_alpha, float4* __restrict__ d_raw, float* __restrict__ d_dir) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int64_t ray = (int64_t)blockIdx.x * kWarps + warp; ray < n_rays; ray += (int64_t)gridDim.x * kWarps) {
     Fwd<C> f;
@@ -179,6 +184,7 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
     }
     float excl = __shfl_down_sync(FULL_MASK, incl, 1);
     if (lane == 31) excl = 0.f;
+    float dnorm = 0.f;
 #pragma unroll
     for (int k = 0; k < C; ++k) {
       int i = base + k;
@@ -187,6 +193,7 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
         float dalpha = G[k] * f.T[k] - suffix / f.q[k];
         if (g_alpha) dalpha += __ldg(g_alpha + ray * S + i);
         float dsig = (f.sig[k] > 0.f) ? dalpha * f.delta[k] * f.e[k] : 0.f;
+        if constexpr (kNorm) dnorm += (f.sig[k] > 0.f) ? dsig * f.sig[k] : dalpha * 0.f;   // 0 * NaN = NaN, as autograd
         float wk = f.w[k];
         float4 o;
         o.x = wk * gR * f.cr[k] * (1.f - f.cr[k]);
@@ -194,6 +201,14 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
         o.z = wk * gB * f.cb[k] * (1.f - f.cb[k]);
         o.w = dsig;
         d_raw[ray * S + i] = o;
+      }
+    }
+    if constexpr (kNorm) {
+      dnorm = warp_sum(dnorm);
+      if (lane == 0) {
+        const float* d = rays_d + ray * d_stride;
+        const float inv2 = norm > 0.f ? 1.f / (norm * norm) : 0.f;
+        for (int c = 0; c < 3; ++c) d_dir[ray * 3 + c] = dnorm * (__ldg(d + c) * inv2);
       }
     }
   }
@@ -367,13 +382,15 @@ composite_fwd4_kernel(const float4* __restrict__ raw, const float* __restrict__ 
 
 // resident blocks per SM: S = 64 is fastest at 4 (64 registers, ~100 B of spills: 78.9 % of the copy peak; 2 blocks / 124
 // registers: 71.5 %), S = 128 at 2 (no spills: 73.4 % against 69.1 % at 4; 3 blocks are worse for both)
-template <int G>
-__global__ void __launch_bounds__(kWarps * 32, (G == 32) ? 2 : 4)
+// (the kNorm variant keeps two blocks per SM at S = 64 as well: with 64 registers it would spill the d |rays_d| sum)
+template <int G, bool kNorm>
+__global__ void __launch_bounds__(kWarps * 32, (G == 32 || kNorm) ? 2 : 4)
 composite_bwd4_kernel(const float4* __restrict__ raw, const float* __restrict__ z, const float* __restrict__ rays_d,
                       int d_stride, const float* __restrict__ noise, int64_t n_rays, int white, int detach_w,
                       const float* __restrict__ g_rgb, const float* __restrict__ g_disp, const float* __restrict__ g_acc,
                       const float* __restrict__ g_depth, const float* __restrict__ g_weights,
-                      const float* __restrict__ g_alpha, float4* __restrict__ d_raw, const MseArgs mse) {
+                      const float* __restrict__ g_alpha, float4* __restrict__ d_raw, const MseArgs mse,
+                      float* __restrict__ d_dir) {
   constexpr int S = 4 * G, RPW = 32 / G;
   const float gs_rgb = (mse.g_sq && mse.target_rgb) ? 2.f * __ldg(mse.g_sq) : 0.f;
   const float gs_disp = (mse.g_sq && mse.target_disp) ? 2.f * __ldg(mse.g_sq + 1) : 0.f;
@@ -435,6 +452,7 @@ composite_bwd4_kernel(const float4* __restrict__ raw, const float* __restrict__ 
     if (sub == G - 1) excl = 0.f;
     // d_raw of this lane's 4 consecutive samples ...
     float4 o[4];
+    float dn = 0.f;   // kNorm: sum of dalpha relu(sigma) delta e over this lane's samples
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       float dalpha = Gk[k] * f.T[k] - (Gw[k] + excl) * rcp_ftz(f.q[k]) + gav[k];
@@ -442,6 +460,19 @@ composite_bwd4_kernel(const float4* __restrict__ raw, const float* __restrict__ 
       o[k].y = f.w[k] * gG * f.cg[k] * (1.f - f.cg[k]);
       o[k].z = f.w[k] * gB * f.cb[k] * (1.f - f.cb[k]);
       o[k].w = (f.sig[k] > 0.f) ? dalpha * f.delta[k] * f.e[k] : 0.f;
+      if constexpr (kNorm) dn += dalpha * fmaxf(f.sig[k], 0.f) * f.delta[k] * f.e[k];   // 0 * NaN = NaN, as autograd
+    }
+    if constexpr (kNorm) {   // d |rays_d| (see composite_bwd_kernel), summed over the ray's group in a fixed order
+      dn = group_sum<G>(dn);
+      if (live_ray && sub == 0) {
+        const float* d = rays_d + ray * d_stride;
+        const float dx = __ldg(d), dy = __ldg(d + 1), dz = __ldg(d + 2);
+        const float n2 = dx * dx + dy * dy + dz * dz;
+        const float inv2 = n2 > 0.f ? 1.f / n2 : 0.f;
+        d_dir[ray * 3 + 0] = dn * (dx * inv2);
+        d_dir[ray * 3 + 1] = dn * (dy * inv2);
+        d_dir[ray * 3 + 2] = dn * (dz * inv2);
+      }
     }
     // ... transposed inside each quad of lanes (lane 4m + j ends up with samples 16m + 4k + j, k = 0..3), so that every store
     // instruction writes 64 contiguous bytes per quad = full 32-byte sectors (16 bytes per lane at a 64-byte stride wrote half
@@ -532,7 +563,8 @@ static int composite_forward_impl(const float* raw, const float* z_vals, const f
 static int composite_backward_impl(const float* raw, const float* z_vals, const float* rays_d, int rays_d_stride,
                                    const float* noise, int64_t n_rays, int n_samples, int white_bkgd, int detach_weights,
                                    const float* g_rgb, const float* g_disp, const float* g_acc, const float* g_depth,
-                                   const float* g_weights, const float* g_alpha, float* d_raw, const MseArgs& mse, void* stream) {
+                                   const float* g_weights, const float* g_alpha, float* d_raw, const MseArgs& mse, float* d_dir,
+                                   void* stream) {
   MVIP_REQUIRE(n_rays == 0 || (raw && z_vals && rays_d && d_raw), MVIP_E_INVALID, "mvip_composite_backward: null pointer");
   MVIP_REQUIRE(n_rays >= 0 && n_samples >= 1 && rays_d_stride >= 3, MVIP_E_INVALID, "mvip_composite_backward: bad shape");
   MVIP_REQUIRE(n_samples <= 512, MVIP_E_UNSUPPORTED, "mvip_composite_backward: n_samples %d > 512", n_samples);
@@ -544,22 +576,30 @@ static int composite_backward_impl(const float* raw, const float* z_vals, const 
   if (vec_ok && (n_samples == 64 || n_samples == 128)) {
     auto* r4 = reinterpret_cast<const float4*>(raw);
     auto* o4 = reinterpret_cast<float4*>(d_raw);
-    if (n_samples == 128)
-      composite_bwd4_kernel<32><<<grid_for_rays4(n_rays, 1), kWarps * 32, 0, (cudaStream_t)stream>>>(
-          r4, z_vals, rays_d, rays_d_stride, noise, n_rays, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth,
-          g_weights, g_alpha, o4, mse);
-    else
-      composite_bwd4_kernel<16><<<grid_for_rays4(n_rays, 2), kWarps * 32, 0, (cudaStream_t)stream>>>(
-          r4, z_vals, rays_d, rays_d_stride, noise, n_rays, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth,
-          g_weights, g_alpha, o4, mse);
+#define MVIP_BWD4(G, NORM)                                                                                                    \
+  composite_bwd4_kernel<G, NORM><<<grid_for_rays4(n_rays, 32 / G), kWarps * 32, 0, (cudaStream_t)stream>>>(                  \
+      r4, z_vals, rays_d, rays_d_stride, noise, n_rays, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth, g_weights, \
+      g_alpha, o4, mse, d_dir)
+    if (n_samples == 128) {
+      if (d_dir) MVIP_BWD4(32, true); else MVIP_BWD4(32, false);
+    } else {
+      if (d_dir) MVIP_BWD4(16, true); else MVIP_BWD4(16, false);
+    }
+#undef MVIP_BWD4
     MVIP_LAUNCH_OK("composite_bwd4_kernel");
     return MVIP_OK;
   }
   MVIP_REQUIRE(!mse.g_sq, MVIP_E_UNSUPPORTED, "mvip_composite_backward_mse: the fused losses need n_samples = 64 or 128 and 16-byte aligned rows");
-  DISPATCH_C(n_samples, (composite_bwd_kernel<C><<<grid_for_rays(n_rays), kWarps * 32, 0, (cudaStream_t)stream>>>(
-                            reinterpret_cast<const float4*>(raw), z_vals, rays_d, rays_d_stride, noise, n_rays,
-                            n_samples, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth, g_weights, g_alpha,
-                            reinterpret_cast<float4*>(d_raw))));
+  if (d_dir)
+    DISPATCH_C(n_samples, (composite_bwd_kernel<C, true><<<grid_for_rays(n_rays), kWarps * 32, 0, (cudaStream_t)stream>>>(
+                              reinterpret_cast<const float4*>(raw), z_vals, rays_d, rays_d_stride, noise, n_rays,
+                              n_samples, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth, g_weights, g_alpha,
+                              reinterpret_cast<float4*>(d_raw), d_dir)));
+  else
+    DISPATCH_C(n_samples, (composite_bwd_kernel<C, false><<<grid_for_rays(n_rays), kWarps * 32, 0, (cudaStream_t)stream>>>(
+                              reinterpret_cast<const float4*>(raw), z_vals, rays_d, rays_d_stride, noise, n_rays,
+                              n_samples, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth, g_weights, g_alpha,
+                              reinterpret_cast<float4*>(d_raw), nullptr)));
   MVIP_LAUNCH_OK("composite_bwd_kernel");
   return MVIP_OK;
 }
@@ -578,7 +618,7 @@ int mvip_composite_backward(const float* raw, const float* z_vals, const float* 
                             const float* g_weights, const float* g_alpha, float* d_raw, void* stream) {
   const MseArgs none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   return composite_backward_impl(raw, z_vals, rays_d, rays_d_stride, noise, n_rays, n_samples, white_bkgd, detach_weights, g_rgb,
-                                 g_disp, g_acc, g_depth, g_weights, g_alpha, d_raw, none, stream);
+                                 g_disp, g_acc, g_depth, g_weights, g_alpha, d_raw, none, nullptr, stream);
 }
 
 size_t mvip_composite_mse_workspace_bytes(void) { return (size_t)(2 * 1184 + 4) * sizeof(float); }
@@ -604,7 +644,20 @@ int mvip_composite_backward_mse(const float* raw, const float* z_vals, const flo
   MVIP_REQUIRE(g_sq && (target_rgb || target_disp), MVIP_E_INVALID, "mvip_composite_backward_mse: null pointer");
   const MseArgs mse = {target_rgb, target_disp, nullptr, nullptr, nullptr, g_sq};
   return composite_backward_impl(raw, z_vals, rays_d, rays_d_stride, noise, n_rays, n_samples, white_bkgd, detach_weights, g_rgb,
-                                 g_disp, g_acc, g_depth, g_weights, g_alpha, d_raw, mse, stream);
+                                 g_disp, g_acc, g_depth, g_weights, g_alpha, d_raw, mse, nullptr, stream);
+}
+
+int mvip_composite_backward_rays(const float* raw, const float* z_vals, const float* rays_d, int rays_d_stride,
+                                 const float* noise, int64_t n_rays, int n_samples, int white_bkgd, int detach_weights,
+                                 const float* target_rgb, const float* target_disp, const float* g_sq, const float* g_rgb,
+                                 const float* g_disp, const float* g_acc, const float* g_depth, const float* g_weights,
+                                 const float* g_alpha, float* d_raw, float* d_rays_d, void* stream) {
+  MVIP_REQUIRE(n_rays == 0 || d_rays_d, MVIP_E_INVALID, "mvip_composite_backward_rays: null d_rays_d");
+  MVIP_REQUIRE(!g_sq == !(target_rgb || target_disp), MVIP_E_INVALID,
+               "mvip_composite_backward_rays: g_sq and a fused-loss target go together");
+  const MseArgs mse = {target_rgb, target_disp, nullptr, nullptr, nullptr, g_sq};
+  return composite_backward_impl(raw, z_vals, rays_d, rays_d_stride, noise, n_rays, n_samples, white_bkgd, detach_weights, g_rgb,
+                                 g_disp, g_acc, g_depth, g_weights, g_alpha, d_raw, mse, d_rays_d, stream);
 }
 
 }  // extern "C"

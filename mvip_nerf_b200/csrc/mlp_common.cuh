@@ -76,4 +76,28 @@ __host__ __device__ inline int mask_word_index(int layer, int r, int h, int ch) 
 
 inline int64_t num_tiles(int64_t n_points) { return (n_points + kTile - 1) / kTile; }
 
+#ifdef __CUDACC__
+// ---- positional encoding (forward encoder and the input-gradient chain) ------------------------
+// sin/cos(x * 2^k): the phase is reduced in "turns" with a two-float product x/(2 pi) (power-of-two
+// scaling and the fractional part are exact), then sin.approx/cos.approx on [-pi, pi].
+__device__ __forceinline__ void pe_axis(float x, int L, float* s, float* c) {
+  const float kInv2PiHi = 0.15915494f;
+  const float kInv2PiLo = 3.0918538e-09f;  // 1/(2 pi) - (double)kInv2PiHi
+  float u_hi = x * kInv2PiHi;
+  float u_lo = fmaf(x, kInv2PiHi, -u_hi) + x * kInv2PiLo;
+  float scale = 1.f;
+#pragma unroll
+  for (int k = 0; k < 10; ++k) {
+    if (k < L) {
+      float a = u_hi * scale;
+      float ph = (a - rintf(a)) + u_lo * scale;
+      float ang = ph * 6.283185307179586f;
+      s[k] = __sinf(ang);
+      c[k] = __cosf(ang);
+      scale *= 2.f;
+    }
+  }
+}
+#endif
+
 }  // namespace mlp

@@ -56,29 +56,6 @@ struct Params {
 // step s: number of 64-wide K chunks of its weight block
 __device__ __forceinline__ int step_nchunks(int s) { return s == 0 ? 1 : ((s == 5 || s == 9) ? 5 : 4); }
 
-// ---- positional encoding ---------------------------------------------------------------------
-// sin/cos(x * 2^k): the phase is reduced in "turns" with a two-float product x/(2 pi) (power-of-two
-// scaling and the fractional part are exact), then sin.approx/cos.approx on [-pi, pi].
-__device__ __forceinline__ void pe_axis(float x, int L, float* s, float* c) {
-  const float kInv2PiHi = 0.15915494f;
-  const float kInv2PiLo = 3.0918538e-09f;  // 1/(2 pi) - (double)kInv2PiHi
-  float u_hi = x * kInv2PiHi;
-  float u_lo = fmaf(x, kInv2PiHi, -u_hi) + x * kInv2PiLo;
-  float scale = 1.f;
-#pragma unroll
-  for (int k = 0; k < 10; ++k) {
-    if (k < L) {
-      float a = u_hi * scale;
-      float ph = (a - rintf(a)) + u_lo * scale;
-      float ang = ph * 6.283185307179586f;
-      s[k] = __sinf(ang);
-      c[k] = __cosf(ang);
-      scale *= 2.f;
-    }
-  }
-}
-
-
 // one half (4 of the 8 sixteen-byte groups) of a PE row; `half` is warp-uniform
 template <int L>
 __device__ __forceinline__ void write_pe_half(uint8_t* img, int row, float x, float y, float z, int half) {

@@ -110,6 +110,142 @@ __global__ void __launch_bounds__(256) rays_pack_kernel(const float* __restrict_
   }
 }
 
+// ---- backward (autograd of the reference's fp32 formulas, in fp32) -------------------------------------------------------------
+// d of one packed row (g[stride]) -> d ro, d rd (through ndc_rays when on) and d v (through v / |v|)
+__device__ __forceinline__ void ray_row_backward(const float* __restrict__ g, const float ro[3], const float rd[3], const float v[3],
+                                                 int use_viewdirs, int voff, const Ndc& ndc, float gro[3], float grd[3], float gv[3]) {
+  if (ndc.on) {
+    const float go0 = g[0], go1 = g[1], go2 = g[2], gd0 = g[3], gd1 = g[4], gd2 = g[5];
+    const float t = -(ndc.near + ro[2]) / rd[2];
+    const float ox = ro[0] + t * rd[0], oy = ro[1] + t * rd[1], oz = ro[2] + t * rd[2];
+    const float rz = 1.f / oz, rz2 = rz * rz;
+    // o_ndc = (sx ox/oz, sy oy/oz, 1 + 2n/oz);  d_ndc = (sx (dx/dz - ox/oz), sy (dy/dz - oy/oz), -2n/oz)
+    const float gox = ndc.sx * (go0 - gd0) * rz;
+    const float goy = ndc.sy * (go1 - gd1) * rz;
+    const float goz = (ndc.sx * ox * (gd0 - go0) + ndc.sy * oy * (gd1 - go1) + ndc.two_near * (gd2 - go2)) * rz2;
+    const float rdz = 1.f / rd[2];
+    grd[0] = ndc.sx * gd0 * rdz;
+    grd[1] = ndc.sy * gd1 * rdz;
+    grd[2] = -(ndc.sx * gd0 * rd[0] + ndc.sy * gd1 * rd[1]) * rdz * rdz;
+    // o' = o + t d;  t = -(n + o.z) / d.z
+    const float gt = gox * rd[0] + goy * rd[1] + goz * rd[2];
+    gro[0] = gox; gro[1] = goy; gro[2] = goz - gt * rdz;
+    grd[0] += t * gox; grd[1] += t * goy; grd[2] += t * goz + gt * (ndc.near + ro[2]) * rdz * rdz;
+  } else {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { gro[k] = g[k]; grd[k] = g[3 + k]; }
+  }
+  gv[0] = gv[1] = gv[2] = 0.f;
+  if (use_viewdirs) {   // v_hat = v / |v|:  d v = (g - v_hat (v_hat . g)) / |v|
+    const float nrm = sqrtf(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
+    const float inv = 1.f / nrm;
+    const float h0 = v[0] * inv, h1 = v[1] * inv, h2 = v[2] * inv;
+    const float gh0 = g[voff], gh1 = g[voff + 1], gh2 = g[voff + 2];
+    const float dot = h0 * gh0 + h1 * gh1 + h2 * gh2;
+    gv[0] = (gh0 - h0 * dot) * inv;
+    gv[1] = (gh1 - h1 * dot) * inv;
+    gv[2] = (gh2 - h2 * dot) * inv;
+  }
+}
+
+__global__ void __launch_bounds__(256) rays_pack_backward_kernel(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
+                                                                 const float* __restrict__ view_d, int64_t n, int use_viewdirs, Ndc ndc,
+                                                                 const float* __restrict__ g_out, float* __restrict__ g_ro,
+                                                                 float* __restrict__ g_rd, float* __restrict__ g_vd) {
+  const int stride = use_viewdirs ? 11 : 8;
+  for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t)gridDim.x * blockDim.x) {
+    float ro[3], rd[3], v[3], gro[3], grd[3], gv[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      ro[k] = rays_o[idx * 3 + k];
+      rd[k] = rays_d[idx * 3 + k];
+      v[k] = view_d ? view_d[idx * 3 + k] : rd[k];
+    }
+    ray_row_backward(g_out + idx * stride, ro, rd, v, use_viewdirs, 8, ndc, gro, grd, gv);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      g_ro[idx * 3 + k] = gro[k];
+      if (view_d) { g_rd[idx * 3 + k] = grd[k]; g_vd[idx * 3 + k] = gv[k]; }
+      else g_rd[idx * 3 + k] = grd[k] + gv[k];
+    }
+  }
+}
+
+// d c2w [3,4] (and d c2w_static) of a pinhole view: per-pixel terms d R[k][m] = d rays_d[k] dir[m], d t = d rays_o, summed per
+// block in a fixed order (thread-strided, then a fixed tree) into partials[block][24]; rays_pose_reduce_kernel adds the blocks
+// in block order.  Entries 0..11: the pose rays_o / rays_d come from, 12..23: the pose of the view directions.
+constexpr int kPoseCap = 148 * 4;
+__global__ void __launch_bounds__(256) rays_pose_backward_kernel(const float* __restrict__ c2w, const float* __restrict__ c2w_static,
+                                                                 int H, int W, float focal, int i0, int j0, int h, int w,
+                                                                 int use_viewdirs, Ndc ndc, const float* __restrict__ g_out,
+                                                                 float* __restrict__ partials) {
+  __shared__ float pose[24];
+  __shared__ float red[8][24];
+  if (threadIdx.x < 12) {
+    pose[threadIdx.x] = c2w[threadIdx.x];
+    pose[12 + threadIdx.x] = c2w_static ? c2w_static[threadIdx.x] : c2w[threadIdx.x];
+  }
+  __syncthreads();
+  const int stride = use_viewdirs ? 11 : 8;
+  const int64_t n = (int64_t)h * w;
+  float acc[24];
+#pragma unroll
+  for (int e = 0; e < 24; ++e) acc[e] = 0.f;
+  for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t)gridDim.x * blockDim.x) {
+    const int i = i0 + (int)(idx / w), j = j0 + (int)(idx % w);
+    const float dir[3] = {__fdiv_rn(__fsub_rn((float)j, __fmul_rn((float)W, .5f)), focal),
+                          -__fdiv_rn(__fsub_rn((float)i, __fmul_rn((float)H, .5f)), focal), -1.f};
+    float ro[3], rd[3], v[3], gro[3], grd[3], gv[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const float* R = pose + 12 + 4 * k;
+      ro[k] = R[3];
+      rd[k] = __fadd_rn(__fadd_rn(__fmul_rn(dir[0], R[0]), __fmul_rn(dir[1], R[1])), __fmul_rn(dir[2], R[2]));
+      const float* Rv = pose + 4 * k;
+      v[k] = __fadd_rn(__fadd_rn(__fmul_rn(dir[0], Rv[0]), __fmul_rn(dir[1], Rv[1])), __fmul_rn(dir[2], Rv[2]));
+    }
+    ray_row_backward(g_out + idx * stride, ro, rd, v, use_viewdirs, 8, ndc, gro, grd, gv);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+#pragma unroll
+      for (int m = 0; m < 3; ++m) {
+        acc[4 * k + m] = fmaf(grd[k], dir[m], acc[4 * k + m]);
+        acc[12 + 4 * k + m] = fmaf(gv[k], dir[m], acc[12 + 4 * k + m]);
+      }
+      acc[4 * k + 3] += gro[k];
+    }
+  }
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int e = 0; e < 24; ++e) {
+    const float s = warp_sum(acc[e]);
+    if (lane == 0) red[warp][e] = s;
+  }
+  __syncthreads();
+  if (threadIdx.x < 24) {
+    float s = 0.f;
+    for (int q = 0; q < 8; ++q) s += red[q][threadIdx.x];
+    partials[(size_t)blockIdx.x * 24 + threadIdx.x] = s;
+  }
+}
+
+// fixed-order sum of the block partials; without a static camera both halves belong to c2w
+__global__ void rays_pose_reduce_kernel(const float* __restrict__ partials, int blocks, float* __restrict__ g_c2w,
+                                        float* __restrict__ g_c2w_static) {
+  const int e = threadIdx.x;
+  __shared__ float tot[24];
+  if (e < 24) {
+    float s = 0.f;
+    for (int b = 0; b < blocks; ++b) s += partials[(size_t)b * 24 + e];
+    tot[e] = s;
+  }
+  __syncthreads();
+  if (e < 12) {
+    if (g_c2w_static) { g_c2w[e] = tot[12 + e]; g_c2w_static[e] = tot[e]; }
+    else g_c2w[e] = tot[e] + tot[12 + e];
+  }
+}
+
 Ndc make_ndc(int on, int H, int W, double focal, double ndc_near) {
   Ndc c{};
   c.on = on ? 1 : 0;
@@ -159,5 +295,45 @@ extern "C" int mvip_rays_pack(const float* rays_o, const float* rays_d, const fl
   rays_pack_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(rays_o, rays_d, view_d, n, near, far, use_viewdirs ? 1 : 0,
                                                                   make_ndc(ndc, H, W, focal, ndc_near), out);
   MVIP_LAUNCH_OK("rays_pack_kernel");
+  return MVIP_OK;
+}
+
+extern "C" size_t mvip_rays_from_pose_backward_workspace_bytes(void) { return (size_t)kPoseCap * 24 * sizeof(float); }
+
+extern "C" int mvip_rays_from_pose_backward(const float* c2w, const float* c2w_static, int H, int W, double focal, int i0, int j0,
+                                            int h, int w, int use_viewdirs, int ndc, double ndc_near, const float* g_out,
+                                            float* g_c2w, float* g_c2w_static, void* workspace, void* stream) {
+  MVIP_REQUIRE(H > 0 && W > 0 && h >= 0 && w >= 0 && i0 >= 0 && j0 >= 0 && i0 + h <= H && j0 + w <= W, MVIP_E_INVALID,
+               "mvip_rays_from_pose_backward: window [%d,+%d) x [%d,+%d) outside the %d x %d image", i0, h, j0, w, H, W);
+  MVIP_REQUIRE(focal != 0., MVIP_E_INVALID, "mvip_rays_from_pose_backward: focal == 0");
+  MVIP_REQUIRE(c2w && g_c2w && workspace && (g_out || (int64_t)h * w == 0), MVIP_E_INVALID,
+               "mvip_rays_from_pose_backward: null pointer");
+  MVIP_REQUIRE(!g_c2w_static == !c2w_static, MVIP_E_INVALID,
+               "mvip_rays_from_pose_backward: c2w_static and g_c2w_static must be given together");
+  const int64_t n = (int64_t)h * w;
+  int64_t blocks = (n + 255) / 256;
+  const int64_t cap = mvip_num_sms() * 4 < kPoseCap ? mvip_num_sms() * 4 : kPoseCap;
+  blocks = blocks < 1 ? 1 : (blocks > cap ? cap : blocks);
+  float* partials = static_cast<float*>(workspace);
+  rays_pose_backward_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+      c2w, c2w_static, H, W, (float)focal, i0, j0, h, w, use_viewdirs ? 1 : 0, make_ndc(ndc, H, W, focal, ndc_near), g_out, partials);
+  MVIP_LAUNCH_OK("rays_pose_backward_kernel");
+  rays_pose_reduce_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(partials, (int)blocks, g_c2w, g_c2w_static);
+  MVIP_LAUNCH_OK("rays_pose_reduce_kernel");
+  return MVIP_OK;
+}
+
+extern "C" int mvip_rays_pack_backward(const float* rays_o, const float* rays_d, const float* view_d, int64_t n, int use_viewdirs,
+                                       int ndc, int H, int W, double focal, double ndc_near, const float* g_out, float* g_rays_o,
+                                       float* g_rays_d, float* g_view_d, void* stream) {
+  MVIP_REQUIRE(n >= 0, MVIP_E_INVALID, "mvip_rays_pack_backward: n < 0");
+  if (n == 0) return MVIP_OK;
+  MVIP_REQUIRE(rays_o && rays_d && g_out && g_rays_o && g_rays_d && (!view_d || g_view_d), MVIP_E_INVALID,
+               "mvip_rays_pack_backward: null pointer");
+  MVIP_REQUIRE(!ndc || (H > 0 && W > 0 && focal != 0.), MVIP_E_INVALID, "mvip_rays_pack_backward: ndc needs H, W, focal");
+  rays_pack_backward_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(rays_o, rays_d, view_d, n, use_viewdirs ? 1 : 0,
+                                                                           make_ndc(ndc, H, W, focal, ndc_near), g_out, g_rays_o,
+                                                                           g_rays_d, g_view_d);
+  MVIP_LAUNCH_OK("rays_pack_backward_kernel");
   return MVIP_OK;
 }

@@ -102,7 +102,7 @@ def render_views_sharded(render_fn, poses, H, W, focal, near, far, normal_k=31, 
     bands with render_fn(H, W, focal, c2w=pose, patch=(i0, 0, n, W), near=, far=, **kwargs) -> [rgb, disp, acc, depth, extras],
     ONE gather of 24 B/pixel brings them to rank 0, which runs the normal-map kernels (a 31 x 31 stencil over the whole
     image; 24 B/pixel of traffic).  Returns on rank 0 a dict of [V,H,W,...] tensors (+ 'normal' [V,3,H,W], mapped to
-    (n + 1) / 2 as in run.py:965); None on the other ranks."""
+    (n + 1) / 2 as in run.py:965); None on the other ranks.  No pose gradients: the gathered images are leaves."""
     from .run_nerf_helpers import depth2normal
     V = len(poses)
     kwargs = {k: v for k, v in kwargs.items() if k not in ("near", "far")}     # bounds merged into the kwargs (run.py:554-559)
@@ -175,7 +175,8 @@ class ShardedGuidanceViews:
                                      # with deferred re-rendering (run._DeferredRays), then one gradient allreduce per network
 
     Communication: one gather (24 B/ray), one scatter (24 B/ray), one 4.77 MB allreduce.  Every rank ends with the full
-    parameter gradient in .grad, exactly as after dist.allreduce_grads in the ray-batch step."""
+    parameter gradient in .grad, exactly as after dist.allreduce_grads in the ray-batch step.  Gradients reach the network
+    parameters only, not the poses: each rank would hold the pose gradient of its own rows, and nothing reduces those."""
 
     def __init__(self, render_kwargs, poses, H, W, focal, near, far, chunk=8192, with_normals=True, normal_k=31):
         from . import run as mrun

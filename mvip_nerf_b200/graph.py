@@ -42,6 +42,9 @@ def default_loss(rgb, disp, acc, depth, extras, target, scale):
 
 
 class GraphedTrainStep:
+    """One CUDA-graph replay per training step.  Gradients reach the network parameters only: the ray batch is copied into the
+    graph's static buffers, so rays or poses that require grad get no gradient here (use the eager render() for that)."""
+
     def __init__(self, render_kwargs_train, optimizer, H, W, focal, n_rays, near=None, far=None, chunk=1024 * 32, loss_fn=default_loss,
                  target_shape=None, warmup=3, device=None, nccl_in_graph=True, overlap_allreduce=False):
         if not torch.cuda.is_available():

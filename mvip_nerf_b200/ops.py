@@ -22,7 +22,9 @@ launch_count = 0
 param_epoch = 0
 _LAUNCHES = {"mvip_rays_from_pose": 1, "mvip_rays_from_pose_ndc": 1, "mvip_rays_pack": 1, "mvip_sample_coarse": 1, "mvip_sample_pdf": 1, "mvip_sample_fine": 1, "mvip_composite_forward": 1,
              "mvip_composite_backward": 1, "mvip_composite_forward_mse": 1, "mvip_composite_backward_mse": 1, "mvip_normal_forward": 2, "mvip_normal_backward": 4, "mvip_normal_forward_xyz": 2, "mvip_normal_backward_xyz": 4, "mvip_embed": 1,
-             "mvip_mlp_pack_weights": 1, "mvip_mlp_forward": 1, "mvip_mlp_backward": 3, "mvip_selftest_umma": 1}
+             "mvip_mlp_pack_weights": 1, "mvip_mlp_forward": 1, "mvip_mlp_backward": 3, "mvip_selftest_umma": 1,
+             "mvip_rays_pack_backward": 1, "mvip_rays_from_pose_backward": 2, "mvip_composite_backward_rays": 1,
+             "mvip_mlp_input_grad": 1}
 
 
 class _KernelTimer:
@@ -126,6 +128,34 @@ def rays_pack(rays_o, rays_d, near, far, use_viewdirs=True, view_d=None, ndc=Fal
     return out
 
 
+def rays_pack_backward(rays_o, rays_d, view_d, g_out, use_viewdirs=True, ndc=False, H=0, W=0, focal=1., ndc_near=1.):
+    """gradient of rays_pack: g_out [n, 8 | 11] -> (d rays_o, d rays_d, d view_d | None), each [n,3]"""
+    rays_o = _f32(rays_o, "rays_o").reshape(-1, 3)
+    rays_d = _f32(rays_d, "rays_d").reshape(-1, 3)
+    view_d = None if view_d is None else _f32(view_d, "view_d").reshape(-1, 3)
+    g_out = _f32(g_out, "g_out")
+    n = rays_d.shape[0]
+    g_o, g_d = torch.empty_like(rays_o), torch.empty_like(rays_d)
+    g_v = None if view_d is None else torch.empty_like(view_d)
+    _call("mvip_rays_pack_backward", _ptr(rays_o), _ptr(rays_d), _ptr(view_d), n, int(bool(use_viewdirs)), int(bool(ndc)), int(H),
+          int(W), float(focal), float(ndc_near), _ptr(g_out), _ptr(g_o), _ptr(g_d), _ptr(g_v), _stream())
+    return g_o, g_d, g_v
+
+
+def rays_from_pose_backward(c2w, c2w_staticcam, H, W, focal, window, g_out, use_viewdirs=True, ndc=False, ndc_near=1.):
+    """gradient of rays_from_pose: g_out [h*w, 8 | 11] -> (d c2w [3,4], d c2w_staticcam [3,4] | None); window = (i0, j0, h, w)"""
+    c2w = _f32(c2w, "c2w")
+    cs = _f32(c2w_staticcam, "c2w_staticcam")
+    g_out = _f32(g_out, "g_out")
+    i0, j0, h, w = [int(v) for v in window]
+    g_c = torch.empty((3, 4), device=c2w.device, dtype=torch.float32)
+    g_cs = None if cs is None else torch.empty((3, 4), device=c2w.device, dtype=torch.float32)
+    ws = torch.empty((_lib.load().mvip_rays_from_pose_backward_workspace_bytes() // 4,), device=c2w.device, dtype=torch.float32)
+    _call("mvip_rays_from_pose_backward", _ptr(c2w), _ptr(cs), int(H), int(W), float(focal), i0, j0, h, w, int(bool(use_viewdirs)),
+          int(bool(ndc)), float(ndc_near), _ptr(g_out), _ptr(g_c), _ptr(g_cs), _ptr(ws), _stream())
+    return g_c, g_cs
+
+
 # ---------------------------------------------------------------------------------------------- sampling
 def sample_coarse(rays, t_vals, t_rand=None, lindisp=False):
     """rays [N,>=8] -> z_vals [N,S]   (run.py:1759-1781)"""
@@ -222,13 +252,22 @@ def composite_forward(raw, z_vals, rays_d, noise=None, white_bkgd=False, need_al
 
 
 def composite_backward(raw, z_vals, rays_d, noise, white_bkgd, detach_weights, g_rgb, g_disp, g_acc, g_depth,
-                       g_weights=None, g_alpha=None, target_rgb=None, target_disp=None, g_sq=None):
+                       g_weights=None, g_alpha=None, target_rgb=None, target_disp=None, g_sq=None, want_rays_d=False):
+    """-> d_raw [N,S,4]; with want_rays_d -> (d_raw, d rays_d [N,3])"""
     raw = _f32(raw, "raw")
     z_vals = _f32(z_vals, "z_vals")
     rays_d, d_stride = _rows3(rays_d, "rays_d")
     N, S = z_vals.shape
     d_raw = torch.empty((N, S, 4), device=raw.device, dtype=torch.float32)
     args = [_f32(t, "grad") for t in (g_rgb, g_disp, g_acc, g_depth, g_weights, g_alpha)]
+    if want_rays_d:
+        fused = g_sq is not None and (target_rgb is not None or target_disp is not None)
+        d_dir = torch.empty((N, 3), device=raw.device, dtype=torch.float32)
+        _call("mvip_composite_backward_rays", _ptr(raw), _ptr(z_vals), _ptr(rays_d), d_stride, _ptr(_f32(noise, "noise")), N, S,
+              int(bool(white_bkgd)), int(bool(detach_weights)), _ptr(_f32(target_rgb, "target_rgb") if fused else None),
+              _ptr(_f32(target_disp, "target_disp") if fused else None), _ptr(_f32(g_sq, "g_sq") if fused else None),
+              *[_ptr(a) for a in args], _ptr(d_raw), _ptr(d_dir), _stream())
+        return d_raw, d_dir
     if g_sq is not None and (target_rgb is not None or target_disp is not None):
         _call("mvip_composite_backward_mse", _ptr(raw), _ptr(z_vals), _ptr(rays_d), d_stride, _ptr(_f32(noise, "noise")), N, S,
               int(bool(white_bkgd)), int(bool(detach_weights)), _ptr(_f32(target_rgb, "target_rgb")), _ptr(_f32(target_disp, "target_disp")),
@@ -395,8 +434,9 @@ class _GradArena:
 grad_arena = _GradArena()
 
 
-def mlp_backward(packed, d_raw, stash, grads=None, accumulate=False):
-    """-> list of 24 fp32 gradient tensors in PARAM_ORDER"""
+def mlp_backward(packed, d_raw, stash, grads=None, accumulate=False, want_workspace=False):
+    """-> list of 24 fp32 gradient tensors in PARAM_ORDER (and the workspace holding this call's dZ images when
+    want_workspace: what mlp_input_grad reads)"""
     lib = _lib.load()
     d_raw = _f32(d_raw, "d_raw").reshape(-1, 4)
     P = d_raw.shape[0]
@@ -420,7 +460,22 @@ def mlp_backward(packed, d_raw, stash, grads=None, accumulate=False):
     else:
         _call("mvip_mlp_backward", _ptr(packed), _ptr(d_raw), P, _ptr(stash), _ptr(ws), arr, int(bool(accumulate)),
               _stream())
-    return grads
+    return (grads, ws) if want_workspace else grads
+
+
+def mlp_input_grad(packed, workspace, rays=None, z_vals=None, viewdir_offset=8, pts=None, dirs=None):
+    """Gradient w.r.t. the MLP's inputs from the dZ images of the mlp_backward call that filled `workspace` (same points).
+    -> d rays [N, ray_stride] (rays mode: o / d / viewdir columns, zeros elsewhere) or (d pts [P,3], d dirs [P,3])"""
+    global launch_count
+    s, keep = _points_struct(rays, z_vals, viewdir_offset, pts, dirs)
+    dev = keep[0].device
+    d6 = torch.empty((s.n_points, 6), device=dev, dtype=torch.float32)
+    d_rays = torch.empty((s.n_rays, s.ray_stride), device=dev, dtype=torch.float32) if rays is not None else None
+    _call("mvip_mlp_input_grad", _ptr(packed), ctypes.byref(s), _ptr(workspace), _ptr(d6), _ptr(d_rays), _stream())
+    if rays is not None:
+        launch_count += 1 if s.n_points > 0 else 0     # the per-ray sum is a second launch
+        return d_rays
+    return d6[:, 0:3], d6[:, 3:6]
 
 
 def selftest_umma(which, a, b):

@@ -111,21 +111,76 @@ def _clip_patch(patch, H, W):
     return i, j, max(0, min(i + len1, H) - i), max(0, min(j + len2, W) - j)
 
 
+def _pose_tensor(x, dev=None):
+    """[3,4] fp32 CUDA view of a pose (numpy or tensor); differentiable torch ops, so a pose that requires grad stays in the graph"""
+    t = torch.as_tensor(x, dtype=torch.float32)
+    dev = dev or (t.device if t.is_cuda else torch.device("cuda", torch.cuda.current_device()))
+    return t.to(dev)[:3, :4].contiguous()
+
+
+class _RaysFromPose(torch.autograd.Function):
+    """ops.rays_from_pose with its backward kernel: d batch -> d c2w (and d c2w_staticcam)"""
+
+    @staticmethod
+    def forward(ctx, c2w, c2w_staticcam, H, W, focal, near, far, use_viewdirs, window, ndc):
+        ctx.save_for_backward(c2w, c2w_staticcam)
+        ctx.cam = (H, W, focal, window, use_viewdirs, ndc)
+        return ops.rays_from_pose(H, W, focal, c2w, near, far, use_viewdirs=use_viewdirs, c2w_staticcam=c2w_staticcam,
+                                  patch=window, ndc=ndc)
+
+    @staticmethod
+    def backward(ctx, g):
+        c2w, cs = ctx.saved_tensors
+        H, W, focal, window, use_viewdirs, ndc = ctx.cam
+        g_c, g_cs = ops.rays_from_pose_backward(c2w, cs, H, W, focal, window or (0, 0, H, W), g, use_viewdirs=use_viewdirs, ndc=ndc)
+        return (g_c, g_cs) + (None,) * 8
+
+
+class _RaysPack(torch.autograd.Function):
+    """ops.rays_pack with its backward kernel: d batch -> d rays_o, d rays_d"""
+
+    @staticmethod
+    def forward(ctx, rays_o, rays_d, near, far, use_viewdirs, ndc, H, W, focal):
+        ctx.save_for_backward(rays_o, rays_d)
+        ctx.cam = (use_viewdirs, ndc, H, W, focal)
+        return ops.rays_pack(rays_o, rays_d, near, far, use_viewdirs=use_viewdirs, ndc=ndc, H=H, W=W, focal=focal)
+
+    @staticmethod
+    def backward(ctx, g):
+        rays_o, rays_d = ctx.saved_tensors
+        use_viewdirs, ndc, H, W, focal = ctx.cam
+        g_o, g_d, _ = ops.rays_pack_backward(rays_o, rays_d, None, g, use_viewdirs=use_viewdirs, ndc=ndc, H=H, W=W, focal=focal)
+        return (g_o.view(rays_o.shape), g_d.view(rays_d.shape)) + (None,) * 7
+
+
+def _needs_grad(*xs):
+    return torch.is_grad_enabled() and any(torch.is_tensor(x) and x.requires_grad for x in xs)
+
+
 def _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch):
     """The ray-batch assembly of render() (run.py:1171-1207) -> (rays_flat [N, 8|9|11|12], sh).
 
     The batch is written by ONE kernel (get_rays / patch / viewdir normalisation / ndc_rays / near / far / cat):
     mvip_rays_from_pose for `c2w=`, mvip_rays_pack for `rays=`.  Only the `depths=` column (used by the out-of-scope sigma
-    loss), non-scalar near / far / focal and `rays=` combined with a static camera take the elementwise torch route."""
+    loss), non-scalar near / far / focal and `rays=` combined with a static camera take the elementwise torch route.
+    When the pose(s) or the given rays require grad, the fused entries run inside autograd Functions whose backward kernels
+    return d c2w / d c2w_staticcam or d rays_o / d rays_d; the torch route is differentiable as it stands."""
     fusable = depths is None and torch.cuda.is_available() and _is_number(near) and _is_number(far) and _is_number(focal)
     if fusable and c2w is not None:
         if patch is not None:
             patch = _clip_patch(patch, H, W)
-        rays_flat = ops.rays_from_pose(H, W, focal, c2w, near, far, use_viewdirs=use_viewdirs, c2w_staticcam=c2w_staticcam,
-                                       patch=patch, ndc=ndc)
+        if _needs_grad(c2w, c2w_staticcam):
+            c = _pose_tensor(c2w)
+            cs = None if c2w_staticcam is None else _pose_tensor(c2w_staticcam, c.device)
+            rays_flat = _RaysFromPose.apply(c, cs, H, W, focal, near, far, use_viewdirs, patch, ndc)
+        else:
+            rays_flat = ops.rays_from_pose(H, W, focal, c2w, near, far, use_viewdirs=use_viewdirs, c2w_staticcam=c2w_staticcam,
+                                           patch=patch, ndc=ndc)
         return rays_flat, ((H, W) if patch is None else (patch[2], patch[3])) + (3,)
     if fusable and c2w is None and (c2w_staticcam is None or not use_viewdirs):
         rays_o, rays_d = rays
+        if _needs_grad(rays_o, rays_d):
+            return _RaysPack.apply(rays_o, rays_d, near, far, use_viewdirs, ndc, H, W, focal), rays_d.shape
         return ops.rays_pack(rays_o, rays_d, near, far, use_viewdirs=use_viewdirs, ndc=ndc, H=H, W=W, focal=focal), rays_d.shape
     if c2w is not None:
         rays_o, rays_d = get_rays(H, W, focal, c2w)
@@ -354,7 +409,8 @@ class _DeferredRays(torch.autograd.Function):
 
     forward  renders every chunk under no_grad (no activation stash: the tensor-bound render kernel);
     backward re-renders one chunk at a time with the stash enabled, back-propagates the slice of the upstream image
-             gradients that belongs to it and accumulates the parameter gradients.
+             gradients that belongs to it and accumulates the parameter gradients; when rays_flat requires grad (a pose or rays
+             that require grad upstream), each chunk's slice is a grad leaf and the slices' gradients are concatenated.
     Peak memory is one chunk's stash (10.3 KB per sample point) instead of the whole view's: 4 x 512 x 512 rays x 192 points
     would need 2 TB, which is why the reference cannot run its guidance views at normalmap_render_factor = 1 (README.md:61).
     The random streams (perturb / raw_noise_std) are replayed by restoring the CUDA generator state, so the re-rendered
@@ -382,8 +438,10 @@ class _DeferredRays(torch.autograd.Function):
             return none
         params = [p for p in ctx.params]
         live = [i for i, p in enumerate(params) if p.requires_grad]
-        if not live:
+        want_rays = ctx.needs_input_grad[0]
+        if not live and not want_rays:
             return none
+        d_rays = []
         dev = ctx.rays.device
         acc = [None] * len(params)
         flat_acc = {}            # first parameter index of a network -> (flat accumulator, its per-parameter views)
@@ -394,10 +452,15 @@ class _DeferredRays(torch.autograd.Function):
                 torch.set_rng_state(ctx.rng)
             for i in range(0, ctx.rays.shape[0], ctx.chunk):
                 with torch.enable_grad():
-                    ret = render_rays(ctx.rays[i:i + ctx.chunk], **ctx.kw)
+                    rays = ctx.rays[i:i + ctx.chunk].detach().requires_grad_(want_rays)
+                    ret = render_rays(rays, **ctx.kw)
                     outs = [ret[k] for k in grads]
                     gs = [grads[k][i:i + ctx.chunk].contiguous() for k in grads]
-                    g = dict(zip(live, torch.autograd.grad(outs, [params[j] for j in live], gs, allow_unused=True)))
+                    wrt = [params[j] for j in live] + ([rays] if want_rays else [])
+                    got = torch.autograd.grad(outs, wrt, gs, allow_unused=True)
+                    g = dict(zip(live, got[:len(live)]))
+                    if want_rays:
+                        d_rays.append(torch.zeros_like(rays) if got[-1] is None else got[-1])
                 for a in range(0, len(params), len(ops.PARAM_ORDER)):
                     # the MLP backward writes a network's 24 gradients back to back: accumulate them as ONE tensor
                     idx = list(range(a, min(a + len(ops.PARAM_ORDER), len(params))))
@@ -419,13 +482,14 @@ class _DeferredRays(torch.autograd.Function):
                     for j, gj in zip(idx, gl):
                         if gj is not None:
                             acc[j] = gj.clone() if acc[j] is None else acc[j].add_(gj)
-        return (None, None, None, None) + tuple(acc)
+        return (torch.cat(d_rays, 0) if want_rays else None, None, None, None) + tuple(acc)
 
 
 def render_deferred(H, W, focal, chunk=1024 * 8, rays=None, c2w=None, ndc=True, near=0., far=1., use_viewdirs=False,
                     c2w_staticcam=None, depths=None, need_alpha=False, detach_weights=False, patch=None, **kwargs):
     """render() with deferred back-propagation: same arguments and return list; rgb / disp / acc / depth (+ rgb0 / disp0 / acc0)
-    carry gradients to the network parameters, the per-sample extras (weights, z_vals, raw, alpha) are detached.
+    carry gradients to the network parameters and, when c2w / c2w_staticcam / rays require grad, to them; the per-sample extras
+    (weights, z_vals, raw, alpha) are detached.
     `chunk` is the number of rays whose activations exist at any one time during backward (default 8192: 16 GB)."""
     if depths is not None:
         raise NotImplementedError("render_deferred: the depths column (sigma loss) is out of scope")

@@ -74,8 +74,9 @@ def get_embedder(multires, i=0):
 # NeRF MLP (run_nerf_helpers.py:74-156)
 # ------------------------------------------------------------------------------------------------
 class _MLPFunction(torch.autograd.Function):
-    """raw = NeRF(PE(pts), PE(dirs)); backward produces parameter gradients only (pts / dirs carry no
-    gradient in the reference's training graph: z_samples is detached, run.py:1812)."""
+    """raw = NeRF(PE(pts), PE(dirs)).  backward gives the parameter gradients and, when the rays / points require grad, their
+    gradient as well (mlp_input_grad, from the dZ images of the same backward): rays mode -> d ray batch (o, d, viewdir
+    columns), points mode -> d pts, d dirs.  z_vals get none: the fine depths are detached in the reference (run.py:1812)."""
 
     @staticmethod
     def forward(ctx, net, mode, a, b, viewdir_offset, need_grad, *params):
@@ -87,6 +88,9 @@ class _MLPFunction(torch.autograd.Function):
             ctx.stash = stash
             ctx.packed = packed
             ctx.net, ctx.pack_gen = net, net._pack_gen
+            ctx.mode, ctx.viewdir_offset = mode, viewdir_offset
+            if ctx.needs_input_grad[2] or ctx.needs_input_grad[3]:
+                ctx.save_for_backward(a, b)   # version-checked: an in-place change before backward raises
         else:
             raw = ops.mlp_forward(packed, **kw)
         ctx.need_grad = need_grad
@@ -103,9 +107,17 @@ class _MLPFunction(torch.autograd.Function):
             # its version-counter error in the same situation)
             raise RuntimeError("NeRF weights were re-packed (optimizer step / load_state_dict / invalidate_packed) between "
                                "this forward and its backward; run backward before changing the parameters")
-        grads = ops.mlp_backward(ctx.packed, d_raw.contiguous(), ctx.stash)
+        want_a, want_b = ctx.needs_input_grad[2], ctx.needs_input_grad[3] and ctx.mode == "points"
+        grads, ws = ops.mlp_backward(ctx.packed, d_raw.contiguous(), ctx.stash, want_workspace=True)
         ctx.stash = None
-        return (None, None, None, None, None, None) + tuple(grads)
+        da = db = None
+        if want_a or want_b:
+            a, b = ctx.saved_tensors
+            if ctx.mode == "rays":
+                da = ops.mlp_input_grad(ctx.packed, ws, rays=a, z_vals=b, viewdir_offset=ctx.viewdir_offset)
+            else:
+                da, db = ops.mlp_input_grad(ctx.packed, ws, pts=a, dirs=b)
+        return (None, None, da if want_a else None, db if want_b else None, None, None) + tuple(grads)
 
 
 class NeRF(nn.Module):
@@ -170,25 +182,30 @@ class NeRF(nn.Module):
         """Call after writing parameters behind torch's back (`.data.copy_`, EMA / weight surgery through raw pointers)."""
         self._packed_key = None
 
-    def _need_grad(self, params):
-        return torch.is_grad_enabled() and any(p.requires_grad for p in params)
+    def _need_grad(self, params, *inputs):
+        """stash for backward when the parameters OR the inputs (rays / points) require grad: a frozen network still
+        back-propagates to its inputs (the full fused backward runs; its parameter gradients are dropped by autograd)"""
+        return torch.is_grad_enabled() and (any(p.requires_grad for p in params) or any(t.requires_grad for t in inputs))
 
     def query_rays(self, ray_batch, z_vals):
         """raw [N,S,4] for pts = o + d*z of every (ray, sample); viewdir = last 3 columns of ray_batch."""
         params = self._ordered_params()
-        raw = _MLPFunction.apply(self, "rays", ray_batch, z_vals, ray_batch.shape[1] - 3, self._need_grad(params), *params)
+        raw = _MLPFunction.apply(self, "rays", ray_batch, z_vals, ray_batch.shape[1] - 3, self._need_grad(params, ray_batch),
+                                 *params)
         return raw.view(z_vals.shape[0], z_vals.shape[1], 4)
 
     def query_points(self, pts, dirs):
-        """raw [P,4] for explicit points / directions ([P,3] each, any row stride)."""
+        """raw [P,4] for explicit points / directions ([P,3] each, any row stride); differentiable w.r.t. pts and dirs."""
         params = self._ordered_params()
-        return _MLPFunction.apply(self, "points", pts, dirs, 0, self._need_grad(params), *params)
+        return _MLPFunction.apply(self, "points", pts, dirs, 0, self._need_grad(params, pts, dirs), *params)
 
     def forward(self, x):
+        """Gradients reach the parameters only, not x: the kernel re-encodes columns 0:3 and 63:66 of x, so the reference's
+        gradient for the other 84 (embedded) columns has no counterpart.  Use query_points for d pts / d dirs."""
         if x.shape[-1] != self.input_ch + self.input_ch_views:
             raise RuntimeError("NeRF.forward expects [..., %d] embedded inputs" % (self.input_ch + self.input_ch_views))
         flat = x.reshape(-1, x.shape[-1])
-        out = self.query_points(flat[:, 0:3], flat[:, self.input_ch:self.input_ch + 3])
+        out = self.query_points(flat[:, 0:3].detach(), flat[:, self.input_ch:self.input_ch + 3].detach())
         return out.reshape(*x.shape[:-1], 4)
 
     def load_weights_from_keras(self, weights):
@@ -305,14 +322,17 @@ class _CompositeFunction(torch.autograd.Function):
         white, detach_w, need_alpha = ctx.flags
         if all(g is None for g in (g_rgb, g_disp, g_acc, g_weights, g_depth, g_alpha, g_sq)):
             return (None,) * 9
-        d_raw = ops.composite_backward(raw, z_vals, rays_d, noise, white, detach_w, g_rgb, g_disp, g_acc, g_depth,
-                                       g_weights, g_alpha if need_alpha else None, target_rgb, target_disp, g_sq)
-        return (d_raw,) + (None,) * 8
+        want_d = ctx.needs_input_grad[2]
+        out = ops.composite_backward(raw, z_vals, rays_d, noise, white, detach_w, g_rgb, g_disp, g_acc, g_depth,
+                                     g_weights, g_alpha if need_alpha else None, target_rgb, target_disp, g_sq, want_rays_d=want_d)
+        d_raw, d_rays_d = out if want_d else (out, None)
+        return (d_raw, None, d_rays_d) + (None,) * 6
 
 
 def raw2outputs(raw, z_vals, rays_d, raw_noise_std=0, white_bkgd=False, pytest=False, need_alpha=False,
                 detach_weights=False, _noise=None, _mse=None):
-    """-> (rgb_map, disp_map, acc_map, weights, depth_map, alpha|None), differentiable w.r.t. raw.
+    """-> (rgb_map, disp_map, acc_map, weights, depth_map, alpha|None), differentiable w.r.t. raw and rays_d (through
+    dists * |rays_d|); z_vals get no gradient.
     `_mse=(target_rgb | None, target_disp | None)` (ours): the squared-error sums of img2mse come out of the same kernels as a
     seventh element sq [2]."""
     noise = _noise
