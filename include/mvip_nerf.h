@@ -78,6 +78,23 @@ int mvip_rays_from_pose_backward(const float* c2w, const float* c2w_static, int 
                                  int w, int use_viewdirs, int ndc, double ndc_near, const float* g_out, float* g_c2w,
                                  float* g_c2w_static, void* workspace, void* stream);
 
+/* Rays of a table of V poses at given pixels: the ray batch of a training step that mixes pixels from many views
+ * (DS_NeRF/run.py:889-908 draws them from all views; here the poses stay differentiable).
+ *   poses   [V,3,4] row-major camera-to-world poses
+ *   pixels  int32 [n,3] = (view, row, col)
+ *   out     [n, 8 + 3*use_viewdirs]: row k is bitwise equal to row row*W + col of mvip_rays_from_pose_ndc(poses[view], NULL, ...)
+ *           over the whole H x W image.  An entry whose view, row or column is out of range gives a row of NaN and reads
+ *           no pose.  No static camera.  One launch, no host synchronisation.
+ * Backward: g_out [n, 8 + 3*use_viewdirs] -> g_poses [V,3,4] (overwritten; views no entry uses get 0, out-of-range entries add
+ *   nothing).  Each view's 12 sums are taken in a fixed order that depends only on `pixels` (no atomics): bitwise reproducible.
+ *   workspace: mvip_rays_from_poses_backward_workspace_bytes(n, V) bytes.  Two launches. */
+int mvip_rays_from_poses(const float* poses, int V, const int* pixels, int64_t n, int H, int W, double focal, float near, float far,
+                         int use_viewdirs, int ndc, double ndc_near, float* out, void* stream);
+size_t mvip_rays_from_poses_backward_workspace_bytes(int64_t n, int V);
+int mvip_rays_from_poses_backward(const float* poses, int V, const int* pixels, int64_t n, int H, int W, double focal,
+                                  int use_viewdirs, int ndc, double ndc_near, const float* g_out, float* g_poses, void* workspace,
+                                  void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Stratified sampling along rays.            replaces DS_NeRF/run.py:1759-1781 (render_rays)
  *   rays    [n_rays, ray_stride] fp32: o(0:3) d(3:6) near(6) far(7) ...

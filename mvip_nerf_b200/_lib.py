@@ -35,6 +35,11 @@ _SIGNATURES = {
     "mvip_rays_from_pose_backward_workspace_bytes": (c_size_t, []),
     "mvip_rays_from_pose_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_int, c_int, c_int, c_int, c_int, c_int,
                                              c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mvip_rays_from_poses": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_double, c_float, c_float, c_int, c_int,
+                                     c_double, c_void_p, c_void_p]),
+    "mvip_rays_from_poses_backward_workspace_bytes": (c_size_t, [c_int64, c_int]),
+    "mvip_rays_from_poses_backward": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_double, c_int, c_int, c_double,
+                                              c_void_p, c_void_p, c_void_p, c_void_p]),
     "mvip_sample_coarse": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "mvip_sample_pdf": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_void_p, c_void_p,
                                 c_void_p, c_void_p]),

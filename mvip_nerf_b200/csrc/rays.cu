@@ -44,6 +44,26 @@ __device__ __forceinline__ void emit_ray(float* __restrict__ o, const float ro[3
   }
 }
 
+// camera-frame direction of pixel (row i, column j): ((j - W/2) / focal, -((i - H/2) / focal), -1)
+__device__ __forceinline__ void pixel_dir(int i, int j, int H, int W, float focal, float dir[3]) {
+  dir[0] = __fdiv_rn(__fsub_rn((float)j, __fmul_rn((float)W, .5f)), focal);
+  dir[1] = -__fdiv_rn(__fsub_rn((float)i, __fmul_rn((float)H, .5f)), focal);
+  dir[2] = -1.f;
+}
+
+// rays_o / rays_d of a direction under pose R, and the view vector under pose Rv ([3,4] row-major each; Rv == R without a
+// static camera)
+__device__ __forceinline__ void pose_ray(const float* R, const float* Rv, const float dir[3], float ro[3], float rd[3], float v[3]) {
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const float* r = R + 4 * k;
+    ro[k] = r[3];
+    rd[k] = __fadd_rn(__fadd_rn(__fmul_rn(dir[0], r[0]), __fmul_rn(dir[1], r[1])), __fmul_rn(dir[2], r[2]));
+    const float* rv = Rv + 4 * k;
+    v[k] = __fadd_rn(__fadd_rn(__fmul_rn(dir[0], rv[0]), __fmul_rn(dir[1], rv[1])), __fmul_rn(dir[2], rv[2]));
+  }
+}
+
 // block-wide: rows of rays [blk, blk + 256) staged in shared memory -> global, consecutive floats per consecutive thread
 __device__ __forceinline__ void flush_rows(const float* rows, float* __restrict__ out, int64_t blk, int64_t n, int stride) {
   __syncthreads();
@@ -70,18 +90,9 @@ __global__ void __launch_bounds__(256) rays_kernel(const float* __restrict__ c2w
     const int64_t idx = blk + threadIdx.x;
     if (idx < n) {
     const int i = i0 + (int)(idx / w), j = j0 + (int)(idx % w);
-    const float dx = __fdiv_rn(__fsub_rn((float)j, __fmul_rn((float)W, .5f)), focal);
-    const float dy = -__fdiv_rn(__fsub_rn((float)i, __fmul_rn((float)H, .5f)), focal);
-    const float dz = -1.f;
-    float ro[3], rd[3], v[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {   // rays_o / rays_d from the (possibly static) camera
-      const float* R = pose + 12 + 4 * k;
-      ro[k] = R[3];
-      rd[k] = __fadd_rn(__fadd_rn(__fmul_rn(dx, R[0]), __fmul_rn(dy, R[1])), __fmul_rn(dz, R[2]));
-      const float* Rv = pose + 4 * k;
-      v[k] = __fadd_rn(__fadd_rn(__fmul_rn(dx, Rv[0]), __fmul_rn(dy, Rv[1])), __fmul_rn(dz, Rv[2]));
-    }
+    float dir[3], ro[3], rd[3], v[3];
+    pixel_dir(i, j, H, W, focal, dir);
+    pose_ray(pose + 12, pose, dir, ro, rd, v);   // rays_o / rays_d from the (possibly static) camera
     emit_ray(rows + threadIdx.x * stride, ro, rd, v, near, far, use_viewdirs, ndc);
     }
     flush_rows(rows, out, blk, n, stride);
@@ -246,6 +257,96 @@ __global__ void rays_pose_reduce_kernel(const float* __restrict__ partials, int 
   }
 }
 
+// rays of a table of poses at given pixels: entry k = (view, row, col) -> row k of the batch, bitwise equal to row row*W + col of
+// rays_kernel's batch of poses[view] over the whole image.  An entry outside [0,V) x [0,H) x [0,W) gives a row of NaN and reads
+// no pose.
+__global__ void __launch_bounds__(256) rays_poses_kernel(const float* __restrict__ poses, int V, const int* __restrict__ pixels,
+                                                         int64_t n, int H, int W, float focal, float near, float far,
+                                                         int use_viewdirs, Ndc ndc, float* __restrict__ out) {
+  __shared__ float rows[256 * 11];
+  const int stride = use_viewdirs ? 11 : 8;
+  for (int64_t blk = (int64_t)blockIdx.x * blockDim.x; blk < n; blk += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t idx = blk + threadIdx.x;
+    if (idx < n) {
+      const int pv = pixels[idx * 3], i = pixels[idx * 3 + 1], j = pixels[idx * 3 + 2];
+      float* o = rows + threadIdx.x * stride;
+      if (pv >= 0 && pv < V && i >= 0 && i < H && j >= 0 && j < W) {
+        const float* P = poses + (int64_t)pv * 12;
+        float dir[3], ro[3], rd[3], v[3];
+        pixel_dir(i, j, H, W, focal, dir);
+        pose_ray(P, P, dir, ro, rd, v);
+        emit_ray(o, ro, rd, v, near, far, use_viewdirs, ndc);
+      } else {
+        for (int e = 0; e < stride; ++e) o[e] = __int_as_float(0x7fc00000);
+      }
+    }
+    flush_rows(rows, out, blk, n, stride);
+  }
+}
+
+// d poses of rays_poses_kernel.  Block b handles view b / chunks and entries [c * kPosesChunk, +kPosesChunk) of the batch,
+// c = b % chunks: each of its entries of that view adds d R[k][m] = (d rays_d[k] + d v[k]) dir[m], d t[k] = d rays_o[k]
+// (thread-strided, then a fixed tree) into partials[b][12]; rays_poses_reduce_kernel adds a view's chunks in chunk order.  So
+// every sum is taken in an order fixed by `pixels` alone, with no atomics.
+// Cost: every block reads the view ids of its whole chunk, so the launch reads V x N ids (4 B each, from L2) besides the N rows
+// it differentiates.  At a training batch (N = 4,096, V = 20: 80 blocks, 0.3 MB of ids) that is noise; it stops being
+// negligible around V x N ~ 1e7 (e.g. 1,000 views x 65,536 rays: 64 M ids, 0.26 GB of L2 reads per step), where a stable
+// sort of the view ids (O(N)) would take its place.
+constexpr int kPosesChunk = 1024;
+__global__ void __launch_bounds__(256) rays_poses_backward_kernel(const float* __restrict__ poses, const int* __restrict__ pixels,
+                                                                  int64_t n, int chunks, int H, int W, float focal,
+                                                                  int use_viewdirs, Ndc ndc, const float* __restrict__ g_out,
+                                                                  float* __restrict__ partials) {
+  __shared__ float red[8][12];
+  const int view = (int)(blockIdx.x / chunks);
+  const int64_t lo = (int64_t)(blockIdx.x % chunks) * kPosesChunk;
+  const int64_t hi = n - lo < kPosesChunk ? n : lo + kPosesChunk;
+  const int stride = use_viewdirs ? 11 : 8;
+  const float* P = poses + (int64_t)view * 12;
+  float acc[12];
+#pragma unroll
+  for (int e = 0; e < 12; ++e) acc[e] = 0.f;
+  for (int64_t idx = lo + threadIdx.x; idx < hi; idx += blockDim.x) {
+    if (pixels[idx * 3] != view) continue;
+    const int i = pixels[idx * 3 + 1], j = pixels[idx * 3 + 2];
+    if (i < 0 || i >= H || j < 0 || j >= W) continue;
+    float dir[3], ro[3], rd[3], v[3], gro[3], grd[3], gv[3];
+    pixel_dir(i, j, H, W, focal, dir);
+    pose_ray(P, P, dir, ro, rd, v);
+    ray_row_backward(g_out + idx * stride, ro, rd, v, use_viewdirs, 8, ndc, gro, grd, gv);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const float gk = grd[k] + gv[k];
+#pragma unroll
+      for (int m = 0; m < 3; ++m) acc[4 * k + m] = fmaf(gk, dir[m], acc[4 * k + m]);
+      acc[4 * k + 3] += gro[k];
+    }
+  }
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int e = 0; e < 12; ++e) {
+    const float s = warp_sum(acc[e]);
+    if (lane == 0) red[warp][e] = s;
+  }
+  __syncthreads();
+  if (threadIdx.x < 12) {
+    float s = 0.f;
+    for (int q = 0; q < 8; ++q) s += red[q][threadIdx.x];
+    partials[(size_t)blockIdx.x * 12 + threadIdx.x] = s;
+  }
+}
+
+// g_poses[v][e] = sum over the view's chunks, in chunk order; views no entry uses get 0
+__global__ void __launch_bounds__(256) rays_poses_reduce_kernel(const float* __restrict__ partials, int64_t V, int chunks,
+                                                                float* __restrict__ g_poses) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= V * 12) return;
+  const int64_t view = t / 12, e = t % 12;
+  float s = 0.f;
+  for (int c = 0; c < chunks; ++c) s += partials[(view * chunks + c) * 12 + e];
+  g_poses[t] = s;
+}
+
 Ndc make_ndc(int on, int H, int W, double focal, double ndc_near) {
   Ndc c{};
   c.on = on ? 1 : 0;
@@ -335,5 +436,47 @@ extern "C" int mvip_rays_pack_backward(const float* rays_o, const float* rays_d,
                                                                            make_ndc(ndc, H, W, focal, ndc_near), g_out, g_rays_o,
                                                                            g_rays_d, g_view_d);
   MVIP_LAUNCH_OK("rays_pack_backward_kernel");
+  return MVIP_OK;
+}
+
+namespace {
+int64_t poses_chunks(int64_t n) { return n <= kPosesChunk ? 1 : (n + kPosesChunk - 1) / kPosesChunk; }
+}  // namespace
+
+extern "C" int mvip_rays_from_poses(const float* poses, int V, const int* pixels, int64_t n, int H, int W, double focal, float near,
+                                    float far, int use_viewdirs, int ndc, double ndc_near, float* out, void* stream) {
+  MVIP_REQUIRE(V >= 0 && n >= 0 && H > 0 && W > 0, MVIP_E_INVALID, "mvip_rays_from_poses: V = %d, N = %lld, image %d x %d", V,
+               (long long)n, H, W);
+  MVIP_REQUIRE(focal != 0., MVIP_E_INVALID, "mvip_rays_from_poses: focal == 0");
+  if (n == 0) return MVIP_OK;
+  MVIP_REQUIRE((poses || V == 0) && pixels && out, MVIP_E_INVALID, "mvip_rays_from_poses: null pointer");
+  rays_poses_kernel<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(poses, V, pixels, n, H, W, (float)focal, near, far,
+                                                                   use_viewdirs ? 1 : 0, make_ndc(ndc, H, W, focal, ndc_near), out);
+  MVIP_LAUNCH_OK("rays_poses_kernel");
+  return MVIP_OK;
+}
+
+extern "C" size_t mvip_rays_from_poses_backward_workspace_bytes(int64_t n, int V) {
+  return (size_t)(V > 0 ? V : 0) * (size_t)poses_chunks(n < 0 ? 0 : n) * 12 * sizeof(float);
+}
+
+extern "C" int mvip_rays_from_poses_backward(const float* poses, int V, const int* pixels, int64_t n, int H, int W, double focal,
+                                             int use_viewdirs, int ndc, double ndc_near, const float* g_out, float* g_poses,
+                                             void* workspace, void* stream) {
+  MVIP_REQUIRE(V >= 0 && n >= 0 && H > 0 && W > 0, MVIP_E_INVALID, "mvip_rays_from_poses_backward: V = %d, N = %lld, image %d x %d",
+               V, (long long)n, H, W);
+  MVIP_REQUIRE(focal != 0., MVIP_E_INVALID, "mvip_rays_from_poses_backward: focal == 0");
+  if (V == 0) return MVIP_OK;
+  MVIP_REQUIRE(poses && g_poses && workspace && (n == 0 || (pixels && g_out)), MVIP_E_INVALID,
+               "mvip_rays_from_poses_backward: null pointer");
+  const int64_t chunks = poses_chunks(n);
+  MVIP_REQUIRE((int64_t)V * chunks < (int64_t)1 << 31, MVIP_E_INVALID, "mvip_rays_from_poses_backward: %d views x %lld chunks", V,
+               (long long)chunks);
+  float* partials = static_cast<float*>(workspace);
+  rays_poses_backward_kernel<<<(unsigned)(V * chunks), 256, 0, (cudaStream_t)stream>>>(
+      poses, pixels, n, (int)chunks, H, W, (float)focal, use_viewdirs ? 1 : 0, make_ndc(ndc, H, W, focal, ndc_near), g_out, partials);
+  MVIP_LAUNCH_OK("rays_poses_backward_kernel");
+  rays_poses_reduce_kernel<<<(unsigned)((V * 12 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(partials, V, (int)chunks, g_poses);
+  MVIP_LAUNCH_OK("rays_poses_reduce_kernel");
   return MVIP_OK;
 }

@@ -24,7 +24,7 @@ _LAUNCHES = {"mvip_rays_from_pose": 1, "mvip_rays_from_pose_ndc": 1, "mvip_rays_
              "mvip_composite_backward": 1, "mvip_composite_forward_mse": 1, "mvip_composite_backward_mse": 1, "mvip_normal_forward": 2, "mvip_normal_backward": 4, "mvip_normal_forward_xyz": 2, "mvip_normal_backward_xyz": 4, "mvip_embed": 1,
              "mvip_mlp_pack_weights": 1, "mvip_mlp_forward": 1, "mvip_mlp_backward": 3, "mvip_selftest_umma": 1,
              "mvip_rays_pack_backward": 1, "mvip_rays_from_pose_backward": 2, "mvip_composite_backward_rays": 1,
-             "mvip_mlp_input_grad": 1}
+             "mvip_mlp_input_grad": 1, "mvip_rays_from_poses": 1, "mvip_rays_from_poses_backward": 2}
 
 
 class _KernelTimer:
@@ -154,6 +154,53 @@ def rays_from_pose_backward(c2w, c2w_staticcam, H, W, focal, window, g_out, use_
     _call("mvip_rays_from_pose_backward", _ptr(c2w), _ptr(cs), int(H), int(W), float(focal), i0, j0, h, w, int(bool(use_viewdirs)),
           int(bool(ndc)), float(ndc_near), _ptr(g_out), _ptr(g_c), _ptr(g_cs), _ptr(ws), _stream())
     return g_c, g_cs
+
+
+def _poses_arg(poses):
+    """[V,3,4] or [V,4,4] fp32 CUDA pose table -> contiguous [V,3,4]"""
+    p = _f32(poses, "poses")
+    if p.dim() != 3 or p.shape[1] not in (3, 4) or p.shape[2] != 4:
+        raise RuntimeError("poses must be [V,3,4] or [V,4,4], got %s" % (tuple(p.shape),))
+    return p[:, :3, :].contiguous()
+
+
+def _pixels_arg(pixels):
+    """[N,3] (view, row, col) CUDA indices, int32 or int64 -> contiguous int32 (int64 values outside int32 stay out of range)"""
+    if not pixels.is_cuda:
+        raise RuntimeError("pixels must be a CUDA tensor: mvip_nerf_b200 has no CPU fallback")
+    if pixels.dim() != 2 or pixels.shape[1] != 3:
+        raise RuntimeError("pixels must be [N,3] = (view, row, col), got %s" % (tuple(pixels.shape),))
+    if pixels.dtype == torch.int64:
+        pixels = pixels.clamp(-1, 2 ** 31 - 1).to(torch.int32)
+    elif pixels.dtype != torch.int32:
+        raise RuntimeError("pixels must be int32 or int64, got %s" % pixels.dtype)
+    return pixels.contiguous()
+
+
+def rays_from_poses(H, W, focal, poses, pixels, near, far, use_viewdirs=True, ndc=False, ndc_near=1.):
+    """pose table [V,3,4] + pixels [N,3] = (view, row, col) -> ray batch [N, 8 | 11]; row k equals row row*W + col of
+    rays_from_pose(poses[view]) over the whole image, bitwise.  Out-of-range entries give rows of NaN."""
+    poses = _poses_arg(poses)
+    pixels = _pixels_arg(pixels)
+    n = pixels.shape[0]
+    out = torch.empty((n, 11 if use_viewdirs else 8), device=pixels.device, dtype=torch.float32)
+    _call("mvip_rays_from_poses", _ptr(poses), poses.shape[0], _ptr(pixels), n, int(H), int(W), float(focal), float(near), float(far),
+          int(bool(use_viewdirs)), int(bool(ndc)), float(ndc_near), _ptr(out), _stream())
+    return out
+
+
+def rays_from_poses_backward(poses, pixels, H, W, focal, g_out, use_viewdirs=True, ndc=False, ndc_near=1.):
+    """gradient of rays_from_poses: g_out [N, 8 | 11] -> d poses [V,3,4] (views no entry uses get 0)"""
+    poses = _poses_arg(poses)
+    pixels = _pixels_arg(pixels)
+    g_out = _f32(g_out, "g_out")
+    V, n = poses.shape[0], pixels.shape[0]
+    g_p = torch.empty((V, 3, 4), device=poses.device, dtype=torch.float32)
+    ws = torch.empty((max(1, _lib.load().mvip_rays_from_poses_backward_workspace_bytes(n, V) // 4),), device=poses.device,
+                     dtype=torch.float32)
+    _call("mvip_rays_from_poses_backward", _ptr(poses), V, _ptr(pixels), n, int(H), int(W), float(focal), int(bool(use_viewdirs)),
+          int(bool(ndc)), float(ndc_near), _ptr(g_out), _ptr(g_p), _ptr(ws), _stream())
+    return g_p
 
 
 # ---------------------------------------------------------------------------------------------- sampling

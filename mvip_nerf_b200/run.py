@@ -136,6 +136,22 @@ class _RaysFromPose(torch.autograd.Function):
         return (g_c, g_cs) + (None,) * 8
 
 
+class _RaysFromPoses(torch.autograd.Function):
+    """ops.rays_from_poses with its backward kernel: d batch -> d poses [V,3,4]"""
+
+    @staticmethod
+    def forward(ctx, poses, pixels, H, W, focal, near, far, use_viewdirs, ndc):
+        ctx.save_for_backward(poses, pixels)
+        ctx.cam = (H, W, focal, use_viewdirs, ndc)
+        return ops.rays_from_poses(H, W, focal, poses, pixels, near, far, use_viewdirs=use_viewdirs, ndc=ndc)
+
+    @staticmethod
+    def backward(ctx, g):
+        poses, pixels = ctx.saved_tensors
+        H, W, focal, use_viewdirs, ndc = ctx.cam
+        return (ops.rays_from_poses_backward(poses, pixels, H, W, focal, g, use_viewdirs=use_viewdirs, ndc=ndc),) + (None,) * 8
+
+
 class _RaysPack(torch.autograd.Function):
     """ops.rays_pack with its backward kernel: d batch -> d rays_o, d rays_d"""
 
@@ -157,14 +173,37 @@ def _needs_grad(*xs):
     return torch.is_grad_enabled() and any(torch.is_tensor(x) and x.requires_grad for x in xs)
 
 
-def _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch):
+def _pose_table_rays(H, W, focal, c2w, pixels, rays, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch):
+    """The `pixels=` form of the ray-batch assembly: c2w [V,3,4] | [V,4,4], pixels [N,3] = (view, row, col) -> ([N, 8|11], sh)"""
+    if c2w is None or rays is not None or c2w_staticcam is not None or depths is not None or patch is not None:
+        raise ValueError("pixels= takes a pose stack c2w [V,3,4] and no rays / c2w_staticcam / depths / patch")
+    if not (_is_number(near) and _is_number(far) and _is_number(focal)):
+        raise NotImplementedError("pixels=: near, far and focal must be scalars (the pose-table ray kernel takes scalars)")
+    t = torch.as_tensor(c2w, dtype=torch.float32)
+    dev = t.device if t.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    if t.dim() != 3:
+        raise ValueError("pixels= needs a pose stack c2w [V,3,4] or [V,4,4], got %s" % (tuple(t.shape),))
+    poses = t.to(dev)[:, :3, :4].contiguous()
+    pixels = torch.as_tensor(pixels, device=dev)
+    if _needs_grad(poses):
+        rays_flat = _RaysFromPoses.apply(poses, pixels, H, W, focal, near, far, use_viewdirs, ndc)
+    else:
+        rays_flat = ops.rays_from_poses(H, W, focal, poses, pixels, near, far, use_viewdirs=use_viewdirs, ndc=ndc)
+    return rays_flat, (pixels.shape[0], 3)
+
+
+def _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch, pixels=None):
     """The ray-batch assembly of render() (run.py:1171-1207) -> (rays_flat [N, 8|9|11|12], sh).
 
     The batch is written by ONE kernel (get_rays / patch / viewdir normalisation / ndc_rays / near / far / cat):
     mvip_rays_from_pose for `c2w=`, mvip_rays_pack for `rays=`.  Only the `depths=` column (used by the out-of-scope sigma
     loss), non-scalar near / far / focal and `rays=` combined with a static camera take the elementwise torch route.
     When the pose(s) or the given rays require grad, the fused entries run inside autograd Functions whose backward kernels
-    return d c2w / d c2w_staticcam or d rays_o / d rays_d; the torch route is differentiable as it stands."""
+    return d c2w / d c2w_staticcam or d rays_o / d rays_d; the torch route is differentiable as it stands.
+    With `pixels` [N,3] = (view, row, col), c2w is a pose stack and mvip_rays_from_poses writes the batch (d stack when it
+    requires grad)."""
+    if pixels is not None:
+        return _pose_table_rays(H, W, focal, c2w, pixels, rays, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch)
     fusable = depths is None and torch.cuda.is_available() and _is_number(near) and _is_number(far) and _is_number(focal)
     if fusable and c2w is not None:
         if patch is not None:
@@ -220,9 +259,12 @@ def _split_outputs(all_ret, sh):
 
 
 def render(H, W, focal, chunk=1024 * 32, rays=None, c2w=None, ndc=True, near=0., far=1., use_viewdirs=False,
-           c2w_staticcam=None, depths=None, need_alpha=False, detach_weights=False, patch=None, **kwargs):
-    """(run.py:1143-1219) -> [rgb_map, disp_map, acc_map, depth_map, extras]."""
-    rays_flat, sh = _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch)
+           c2w_staticcam=None, depths=None, need_alpha=False, detach_weights=False, patch=None, pixels=None, **kwargs):
+    """(run.py:1143-1219) -> [rgb_map, disp_map, acc_map, depth_map, extras].
+    `pixels` (ours) [N,3] int = (view, row, col): c2w is then a pose stack [V,3,4] | [V,4,4], the batch is those N pixels of
+    their views (a training batch drawn from many views, run.py:889-908), the maps are [N, ...], and a stack that requires grad
+    gets d stack."""
+    rays_flat, sh = _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, depths, patch, pixels)
     all_ret = batchify_rays(rays_flat, chunk, need_alpha=need_alpha, detach_weights=detach_weights, **kwargs)
     return _split_outputs(all_ret, sh)
 
@@ -486,14 +528,14 @@ class _DeferredRays(torch.autograd.Function):
 
 
 def render_deferred(H, W, focal, chunk=1024 * 8, rays=None, c2w=None, ndc=True, near=0., far=1., use_viewdirs=False,
-                    c2w_staticcam=None, depths=None, need_alpha=False, detach_weights=False, patch=None, **kwargs):
-    """render() with deferred back-propagation: same arguments and return list; rgb / disp / acc / depth (+ rgb0 / disp0 / acc0)
-    carry gradients to the network parameters and, when c2w / c2w_staticcam / rays require grad, to them; the per-sample extras
+                    c2w_staticcam=None, depths=None, need_alpha=False, detach_weights=False, patch=None, pixels=None, **kwargs):
+    """render() with deferred back-propagation: same arguments (pixels= included) and return list; rgb / disp / acc / depth (+ rgb0 /
+    disp0 / acc0) carry gradients to the network parameters and, when c2w / c2w_staticcam / rays require grad, to them; the per-sample extras
     (weights, z_vals, raw, alpha) are detached.
     `chunk` is the number of rays whose activations exist at any one time during backward (default 8192: 16 GB)."""
     if depths is not None:
         raise NotImplementedError("render_deferred: the depths column (sigma loss) is out of scope")
-    rays_flat, sh = _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, None, patch)
+    rays_flat, sh = _assemble_rays(H, W, focal, rays, c2w, ndc, near, far, use_viewdirs, c2w_staticcam, None, patch, pixels)
     kw = dict(kwargs, need_alpha=need_alpha, detach_weights=detach_weights)
     params = [p for _, ps in _net_params(kwargs) for p in ps]
     holder = {}
